@@ -29,6 +29,7 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -36,6 +37,9 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the tree may be read-only: no __pycache__ next to the imported modules
+# seeded frames take tens of seconds to generate: cached per user in the temporary directory, never in the tree
+FRAME_CACHE = os.path.join(tempfile.gettempdir(), f"fast_livo2_b200_frames_{os.getuid()}")
 
 METRIC = "ESIKF update iters/sec @100k LiDAR pts+2k patches"
 UNIT = "iters/s"
@@ -56,7 +60,13 @@ def parse_args():
     ap.add_argument("--no-shim", action="store_true", help="skip the e2e_shim leg")
     ap.add_argument("--comm", default="p2p", choices=["p2p", "nccl"], help="N>1: in-kernel NVLink peer-memory exchange (default) or NCCL per iteration")
     ap.add_argument("--tuning", type=int, default=0, help="esikf_set_tuning flags (1: stage plane records with __ldg copies instead of cp.async.bulk)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (posterior states, iteration statistics, per-point association and per-patch "
+                         "errors) to DIR/<name>.npy, float64 / float32, for comparing two builds on the same seeded inputs")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    return args
 
 
 # ----------------------------------------------------------------------------------------------------------------------
@@ -64,7 +74,7 @@ def make_workload(args):
     from fast_livo2_b200 import workloads as W
 
     t0 = time.time()
-    fr = W.frame(args.config)
+    fr = W.frame(args.config, cache_dir=FRAME_CACHE)
     fr["gen_seconds"] = time.time() - t0
     return fr
 
@@ -143,7 +153,7 @@ def ncu_traffic():
 # ---------------------------------------------------------------------------------------------------------------------- CPU oracle legs
 def native_baseline_build():
     """Build liborc_baseline.so ON THIS HOST (-march=native must mean the machine the number is taken on). Returns the path or None."""
-    out_dir = os.path.join("/tmp", f"orc_native_{os.getuid()}")
+    out_dir = os.path.join(tempfile.gettempdir(), f"orc_native_{os.getuid()}")
     os.makedirs(out_dir, exist_ok=True)
     so = os.path.join(out_dir, "liborc_baseline.so")
     src = [os.path.join(ROOT, "oracle", f) for f in ("orc_lio.cpp", "orc_vio.cpp", "orc_capi.cpp")]
@@ -205,6 +215,25 @@ def state_error(s, ref):
     d = np.sqrt(np.abs(np.diag(b["cov"])))
     cov = float((np.abs(a["cov"] - b["cov"]) / np.maximum(np.outer(d, d), 1e-300)).max())
     return {"rot_rad": rot, "pos_rel": pos, "rest_rel": rest, "cov_rel_per_element": cov}
+
+
+def dump_outputs(out_dir, rl, vl, per_point):
+    """What a caller of the timed path (esikf_lio_run + esikf_lio_fetch, esikf_vio_run + esikf_vio_fetch) receives for the last
+    timed step, one DIR/<name>.npy per array; integer outputs are stored as float64 (exact). The largest workload (cfg5:
+    300 k points, 4 k patches) writes about 6 MB."""
+    arrays = {"lio_state": rl["state"], "lio_iters": [rl["iters"]], "lio_matched_points": rl["M"], "lio_total_residual": rl["total_residual"],
+              "lio_converged": rl["converged"]}
+    if per_point:
+        arrays.update(lio_match_plane=rl["match_plane"], lio_normal_plane=rl["normal_plane"], lio_dis_to_plane=rl["dis_to_plane"])
+    if vl is not None:
+        arrays.update(vio_state=vl["state"], vio_total_iters=[vl["total_iters"]], vio_iters_per_level=vl["iters_per_level"],
+                      vio_accepted_per_level=vl["accepted_per_level"])
+        if per_point:
+            arrays["vio_errors"] = vl["errors"]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        np.save(os.path.join(out_dir, f"{name}.npy"), a if a.dtype in (np.float32, np.float64) else a.astype(np.float64))
 
 
 def parity_block(fr, r0, v0, world):
@@ -548,8 +577,11 @@ def b200_arm(args, rank, world, local_rank):
         dist.all_reduce(stat, op=dist.ReduceOp.MAX)
     total_ms, med_ms, max_ms = (float(x) for x in stat.tolist())
     # the last timed update must reproduce the first bit for bit (same inputs, deterministic reduction order)
-    vl = ctx.vio_fetch(errors=False) if has_vio else None
-    rl = ctx.lio_fetch(per_point=False)
+    per_point = args.dump_outputs is not None and world == 1  # a rank of a sharded run holds only its slice of the per-point outputs
+    vl = ctx.vio_fetch(errors=per_point) if has_vio else None
+    rl = ctx.lio_fetch(per_point=per_point)
+    if args.dump_outputs is not None and rank == 0:
+        dump_outputs(args.dump_outputs, rl, vl, per_point)
     same = rl["iters"] == r0["iters"] and rl["M"].tolist() == r0["M"].tolist()
     if has_vio:
         same = same and vl["total_iters"] == v0["total_iters"] and np.array_equal(vl["state"], v0["state"])

@@ -43,11 +43,12 @@ def describe(name):
     return dict(workload=d, named_gpus=gpus)
 
 
-def frame(name, **override):
-    """The seeded frame of a named config (pickle-cached under .frame_cache/); keyword overrides replace generator arguments."""
+def frame(name, cache_dir=None, **override):
+    """The seeded frame of a named config (pickle-cached under cache_dir, default .frame_cache/); keyword overrides replace
+    generator arguments."""
     d, gpus, kw = _spec(name)
     kw = dict(kw, **override)
-    fr = S.cached_frame(**kw)
+    fr = S.cached_frame(cache_dir=cache_dir, **kw)
     fr.setdefault("vis_pos", [])
     fr["workload"] = d
     fr["named_gpus"] = gpus

@@ -66,15 +66,56 @@ class HostMap:
         return dict(nodes=int(u[0]), recs=int(u[1]), pool_points=int(u[2]), roots=int(u[3]))
 
 
-def compare_flat_maps(a, b, rtol=1e-9, what=("a", "b"), exact=False):
+def _by_key(flat):
+    """Roots sorted by key, their candidate counts and candidate records in that order."""
+    keys = np.asarray(flat["keys"]).reshape(-1, 3)
+    order = np.lexsort(keys.T[::-1])
+    count = np.asarray(flat["count"])[order]
+    sel = np.concatenate([np.arange(f, f + c) for f, c in zip(np.asarray(flat["first"])[order], count)] or [np.zeros(0, np.int64)]).astype(np.int64)
+    return keys[order], count, flat["planes"][sel]
+
+
+def _structure_digest(keys, count, planes):
+    from parity_util import digest
+
+    return "/".join(digest(a) for a in (keys, count, planes["layer"], planes["path"]))
+
+
+def map_record(flat, n_roots, seed):
+    """A flattened map reduced to what a golden file can hold: a digest of its whole structure (root keys, candidates per root,
+    layer / path of every candidate) and the complete records of a seeded sample of `n_roots` roots that hold planes
+    (compare_map_record)."""
+    keys, count, planes = _by_key(flat)
+    held = np.nonzero(count > 0)[0]
+    pick = np.sort(np.random.default_rng(seed).choice(held, min(n_roots, len(held)), replace=False))
+    start = np.concatenate([[0], np.cumsum(count)[:-1]]).astype(np.int64)
+    sel = np.concatenate([np.arange(start[i], start[i] + count[i]) for i in pick]).astype(np.int64)
+    return dict(structure=np.str_(_structure_digest(keys, count, planes)), keys=keys[pick], count=count[pick].astype(np.int32),
+                first=np.concatenate([[0], np.cumsum(count[pick])[:-1]]).astype(np.int32), planes=planes[sel])
+
+
+def compare_map_record(flat, rec, rtol=1e-9, what=("a", "b")):
+    """compare_flat_maps against a map_record: the structure of the whole map bit for bit, the sampled roots' plane records
+    within the tolerances of compare_flat_maps. Returns the number of planes in the map."""
+    keys, count, planes = _by_key(flat)
+    assert _structure_digest(keys, count, planes) == str(rec["structure"]), f"root voxels, candidate counts or candidate order differ between {what[0]} and {what[1]}"
+    compare_flat_maps(flat, dict(keys=rec["keys"], first=rec["first"], count=rec["count"], planes=rec["planes"]), rtol=rtol, what=what, subset=True)
+    return len(planes)
+
+
+def compare_flat_maps(a, b, rtol=1e-9, what=("a", "b"), exact=False, subset=False):
     """Same root keys, same candidate count per root, candidate j of a root = the same plane (centre, +-normal, plane_var, d,
     radius, layer, path) within rtol. Returns the number of planes compared. The eigenvector sign of a fit is free: a flipped
-    normal flips d and the normal-position cross block of plane_var."""
+    normal flips d and the normal-position cross block of plane_var. subset: b holds some of a's roots, only those are compared."""
     ka = {tuple(k): i for i, k in enumerate(a["keys"].tolist())}
     kb = {tuple(k): i for i, k in enumerate(b["keys"].tolist())}
-    assert set(ka) == set(kb), f"root voxels differ: {len(set(ka) - set(kb))} only in {what[0]}, {len(set(kb) - set(ka))} only in {what[1]}"
-    ia = np.array([ka[k] for k in ka], np.int64)
-    ib = np.array([kb[k] for k in ka], np.int64)
+    if subset:
+        assert set(kb) <= set(ka), f"{len(set(kb) - set(ka))} root voxels of {what[1]} missing in {what[0]}"
+    else:
+        assert set(ka) == set(kb), f"root voxels differ: {len(set(ka) - set(kb))} only in {what[0]}, {len(set(kb) - set(ka))} only in {what[1]}"
+    common = list(kb) if subset else list(ka)
+    ia = np.array([ka[k] for k in common], np.int64)
+    ib = np.array([kb[k] for k in common], np.int64)
     assert np.array_equal(a["count"][ia], b["count"][ib]), "candidate counts per root differ"
     sel_a = np.concatenate([np.arange(f, f + c) for f, c in zip(a["first"][ia], a["count"][ia])] or [np.zeros(0, np.int64)]).astype(np.int64)
     sel_b = np.concatenate([np.arange(f, f + c) for f, c in zip(b["first"][ib], b["count"][ib])] or [np.zeros(0, np.int64)]).astype(np.int64)

@@ -41,6 +41,22 @@ def rel(a, b):
     return float(np.abs(a - b).max() / max(np.abs(b).max(), 1e-300))
 
 
+def digest(a):
+    """SHA-256 of an array's shape and values, for bit-exact comparisons with stored outputs too large to commit in full.
+    Floats are widened to float64 (exact) with -0.0 folded into 0.0, integers to int64: for arrays without NaN, equal digests <=> np.array_equal."""
+    import hashlib
+
+    a = np.asarray(a)
+    a = np.ascontiguousarray(a.astype(np.float64) + 0.0 if a.dtype.kind == "f" else a.astype(np.int64))
+    return hashlib.sha256(repr(a.shape).encode() + a.tobytes()).hexdigest()
+
+
+def load_golden(path, prefix):
+    """The record stored under `prefix.` in a golden .npz (keys `prefix.field`), as {field: array}."""
+    with np.load(path, allow_pickle=False) as g:
+        return {k[len(prefix) + 1:]: g[k] for k in g.files if k.startswith(prefix + ".")}
+
+
 def edge_scan(fr, seed=4):
     """World-frame points where the voxel indexing and the neighbour rule of BuildResidualListOMP (src/voxel_map.cpp:665-691)
     are fragile, for a frame's map (identity pose and extrinsics, so p_w is the float point itself):
