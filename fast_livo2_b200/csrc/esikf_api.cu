@@ -968,6 +968,10 @@ int esikf_vio_set_image(esikf_ctx *ctx, const uint8_t *img, int32_t width, int32
 int esikf_vio_set_patches(esikf_ctx *ctx, const double *pos, const float *warp_patch, const int32_t *search_levels, const double *inv_expo_list, int32_t n) {
   if (!ctx || n < 0 || (n > 0 && (!pos || !warp_patch || !search_levels || !inv_expo_list))) return fail(ctx, ESIKF_ERR_ARG, "vio_set_patches: bad argument");
   if (!ctx->have_cam) return fail(ctx, ESIKF_ERR_STATE, "vio_set_patches before vio_set_camera");
+  // the kernels shift by the tap stride 1 << (level + search_level) and index the per-stride tensor maps with it: same range
+  // as warp_affine, checked before anything is uploaded so the installed patches stay as they were
+  for (int i = 0; i < n; i++)
+    if (search_levels[i] < 0 || search_levels[i] > 8) return fail(ctx, ESIKF_ERR_ARG, "vio_set_patches: search level %d of patch %d", search_levels[i], i);
   CK(cudaSetDevice(ctx->device));
   const int L = ctx->vio_cfg.patch_pyrimid_level;
   CK(ctx->vis_pos.reserve((size_t)n * 3 + 4));

@@ -96,6 +96,11 @@ fr = _inputs("distorted_pinhole")[0]
 rows = list(V.patch_producer_calls(O.RefVIO(fr["cam_cfg"], fr["ext"], fr["vio_cfg"])))
 put(vio, "patch", dict(A=np.stack([a for a, _, _, _ in rows]), search_level=np.array([s for _, s, _, _ in rows], np.int32),
                        warp_affine=np.array([wd for _, _, wd, _ in rows]), image_patch=np.array([p for _, _, _, p in rows])))
+b, prior, _, centres = V.edge_wrap_inputs()
+rv = O.RefVIO(b["cam_cfg"], b["ext"], b["vio_cfg"])
+r = rv.update(b["img"], b["vis_pos"], b["warp_patch"], b["search_levels"], b["inv_ref_expo"], prior, prior)
+put(vio, "edge_wrap", dict(state=r["state"], errors=r["errors"], warp_patch=np.str_(digest(b["warp_patch"])), search_levels=b["search_levels"],
+                           image_patch=V.edge_wrap_image_patches(rv, b["img"], centres, b["vio_cfg"].levels)))
 from fast_livo2_b200 import workloads as W  # noqa: E402
 
 for name, (_, want_vio) in V.BASELINE_COUNTS.items():

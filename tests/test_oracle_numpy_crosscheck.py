@@ -342,3 +342,45 @@ def test_numpy_restatement_of_the_inverse_compositional_variant(small_vio_frame)
     vio.set_inverse(False)
     fwd = vio.update(fr["img"], pos, wp, np.zeros(n, np.int32), np.ones(n), fr["state_prior"], fr["state_prior"])
     assert fwd["HTH"][level][0][6, 6] > 0  # the forward variant is untouched by the switch
+
+
+def _numpy_image_patch(img, pc, level):
+    """getImagePatch (vio.cpp:203-225) with the oracle's border rule written out: raw linear indices v * width + u (left /
+    right overhangs wrap to the neighbouring row) and 0 where the index leaves [0, width * height) (DESIGN §4)."""
+    h, w = img.shape
+    flat = img.reshape(-1)
+    s = 1 << level
+    u_ref, v_ref = f32(pc[0]), f32(pc[1])
+    ui = int(np.floor(f32(pc[0] / s)) * f32(s))
+    vi = int(np.floor(f32(pc[1] / s)) * f32(s))
+    su, sv = (u_ref - f32(ui)) / f32(s), (v_ref - f32(vi)) / f32(s)
+    wtl, wtr = f32((1.0 - float(su)) * (1.0 - float(sv))), f32(float(su) * (1.0 - float(sv)))
+    wbl, wbr = f32((1.0 - float(su)) * float(sv)), su * sv
+    pix = lambda i: f32(flat[i]) if 0 <= i < w * h else f32(0)
+    out = np.zeros(64, f32)
+    for x in range(8):
+        base = (vi - 4 * s + x * s) * w + (ui - 4 * s)
+        for y in range(8):
+            b = base + y * s
+            out[x * 8 + y] = wtl * pix(b) + wtr * pix(b + s) + wbl * pix(b + s * w) + wbr * pix(b + s * w + s)
+    return out
+
+
+def test_numpy_restatement_of_image_patch_at_the_border(small_vio_frame):
+    """Centres whose footprints wrap left / right and leave the buffer above / below, at every level: the oracle's pix()
+    rule bit for bit. The reference source pins the in-buffer wrap (test_oracle_ref_pin_vio); this pins the 0 outside."""
+    from parity_util import border_pixels
+
+    fr = small_vio_frame
+    cam = fr["cam_cfg"]
+    vio = O.OracleVIO(cam, fr["ext"], fr["vio_cfg"])
+    px = border_pixels(cam, fr["vio_cfg"].levels, seed=3)[0]
+    px = np.concatenate([px, [[-3.5, -2.25], [cam.width + 2.75, cam.height + 1.5], [0.0, 0.0]]])
+    n_outside = 0
+    for level in range(fr["vio_cfg"].levels):
+        s = 1 << level
+        for c in px:
+            want = _numpy_image_patch(fr["img"], c, level)
+            assert np.array_equal(vio.get_image_patch(fr["img"], c, level), want), (level, c)
+            n_outside += (np.floor(c[1] / s) * s - 4 * s) * cam.width + np.floor(c[0] / s) * s - 4 * s < 0
+    assert n_outside > 20

@@ -131,6 +131,50 @@ def test_oracle_matches_reference_vio_golden():
         np.testing.assert_allclose(orc["errors"], g[f"{name}_errors"], rtol=1e-6, atol=1e-4)
 
 
+def edge_wrap_inputs():
+    """The "small" frame with visual points whose tap footprints cross the LEFT and RIGHT image edges at every tap stride
+    1 .. 32 (parity_util.border_frame: one stride inside, on the edge column, one stride past, half outside), rows kept to
+    h/2 +- 50. There the reference's raw linear-index reads (img.data + v * width + u) wrap to the neighbouring row, which is
+    defined behaviour as long as every index stays inside [0, width * height): asserted here for every patch at every
+    pyramid level at the prior and at the oracle's posterior, with 8 rows to spare for the iterates in between. Returns
+    (frame, prior, oracle update, getImagePatch centres)."""
+    from parity_util import border_frame, tap_origin
+
+    fr = get_frame(**CASES["small"])
+    prior = _prior(fr)
+    cam, L = fr["cam_cfg"], fr["vio_cfg"].levels
+    b = border_frame(fr, prior, seed=21, n_interior=0, edges=("left", "right"), corners=False, outside=False, rows=(cam.height / 2 - 50, cam.height / 2 + 50))
+    o = O.OracleVIO(cam, fr["ext"], fr["vio_cfg"]).update(b["img"], b["vis_pos"], b["warp_patch"], b["search_levels"], b["inv_ref_expo"], prior, prior)
+    w, h = cam.width, cam.height
+    crosses = np.zeros(len(b["vis_pos"]), bool)
+    for state in (prior, o["state"]):
+        for level in range(L):
+            s = 1 << (level + b["search_levels"].astype(np.int64))
+            x0, y0 = tap_origin(cam, fr["ext"], state, b["vis_pos"], s)
+            assert np.all(y0 * w + x0 >= 8 * w) and np.all((y0 + 10 * s) * w + x0 + 10 * s < (h - 8) * w), "a footprint leaves the buffer"
+            crosses |= (x0 < 0) | (x0 + 10 * s >= w)
+    assert crosses.mean() > 0.5
+    return b, prior, o, b["bp_px"]
+
+
+def edge_wrap_image_patches(vio, img, centres, levels):
+    """Digests of getImagePatch at every pyramid level for centres on the left / right edges (wrapping footprints)."""
+    return np.array([[digest(vio.get_image_patch(img, c, lvl)) for lvl in range(levels)] for c in centres])
+
+
+def test_oracle_reproduces_the_reference_source_where_footprints_wrap_rows():
+    """Left / right border footprints at tap strides up to 32: the oracle's linear-index reads (pix()) against the reference
+    source's raw img.data reads, through the whole update and through getImagePatch."""
+    b, prior, orc, centres = edge_wrap_inputs()
+    ref = load_golden(PINS, "edge_wrap")
+    assert digest(b["warp_patch"]) == ref["warp_patch"] and np.array_equal(b["search_levels"], ref["search_levels"])
+    assert orc["total_iters"] >= 4
+    assert_state_close(orc["state"], ref["state"], rot_tol=1e-11, pos_tol=1e-11, cov_tol=1e-9, rest_tol=1e-11)
+    np.testing.assert_allclose(orc["errors"], ref["errors"], rtol=1e-6, atol=1e-4)
+    vio = O.OracleVIO(b["cam_cfg"], b["ext"], b["vio_cfg"])
+    assert (edge_wrap_image_patches(vio, b["img"], centres, b["vio_cfg"].levels) == ref["image_patch"]).all()
+
+
 BASELINE_COUNTS = {  # per-iteration matched points / VIO iterations the CUDA bench lines report for these frames (profiles/bench_r02_*)
     "cfg2": ([99663, 99869, 99883, 99892, 99896], 18),
     "cfg3": (None, -1),  # HILTI fisheye + corridor scene: no CUDA bench line this round, the pin itself is what is checked
