@@ -60,9 +60,21 @@ static NcclApi g_nccl;
 enum { NCCL_FLOAT64 = 8, NCCL_SUM = 0 };
 
 // ---------------------------------------------------------------------------------------------------------------------
+// Device array that owns its memory: grows (contents discarded) on reserve, freed with its owner.
 template <typename T> struct DevBuf {
   T *p = nullptr;
   size_t cap = 0;
+  DevBuf() = default;
+  DevBuf(const DevBuf &) = delete;
+  DevBuf &operator=(const DevBuf &) = delete;
+  DevBuf(DevBuf &&o) noexcept : p(o.p), cap(o.cap) { o.p = nullptr, o.cap = 0; }
+  DevBuf &operator=(DevBuf &&o) noexcept {
+    std::swap(p, o.p), std::swap(cap, o.cap);
+    return *this;
+  }
+  ~DevBuf() {
+    if (p) cudaFree(p);
+  }
   cudaError_t reserve(size_t n) {
     if (n <= cap) return cudaSuccess;
     if (p) cudaFree(p);
@@ -72,11 +84,58 @@ template <typename T> struct DevBuf {
     if (e == cudaSuccess) cap = want;
     return e;
   }
-  void release() {
-    if (p) cudaFree(p);
-    p = nullptr, cap = 0;
+  // reserve `reserve_n` elements, then copy the first `n` from the host on `st` (nothing when n == 0)
+  cudaError_t upload(const T *src, size_t n, size_t reserve_n, cudaStream_t st) {
+    cudaError_t e = reserve(reserve_n);
+    if (e == cudaSuccess && n) e = cudaMemcpyAsync(p, src, n * sizeof(T), cudaMemcpyHostToDevice, st);
+    return e;
   }
 };
+
+// One arena of the device-resident voxel map. The context holds two: esikf_map_device_slide copies the surviving roots
+// into the spare one, then the two change roles. A host-uploaded map (esikf_map_upload) uses slots, planes and recs only.
+struct MapStorage {
+  DevBuf<HashSlot> slots;
+  DevBuf<int> slot_root, slot_cap;
+  DevBuf<MapNode> nodes;
+  DevBuf<double> pool;
+  DevBuf<PlaneRec> recs;        // what the residual kernel reads (144-byte records derived on the device)
+  DevBuf<esikf_plane> planes;   // the map as uploaded / refitted (256-byte records)
+  DevBuf<int> rec_node, counters;
+  DevBuf<unsigned long long> counters64;
+  uint32_t hash_cap = 0;
+  int node_cap = 0, rec_cap = 0;
+  long long pool_cap = 0;
+  cudaError_t reserve(uint32_t hashes, int nodes_n, int recs_n, long long points) {
+    cudaError_t e;
+    if ((e = slots.reserve(hashes)) || (e = slot_root.reserve(hashes)) || (e = slot_cap.reserve(hashes)) || (e = nodes.reserve((size_t)nodes_n)) ||
+        (e = pool.reserve((size_t)points * MAP_PT_D)) || (e = recs.reserve((size_t)recs_n)) || (e = planes.reserve((size_t)recs_n)) ||
+        (e = rec_node.reserve((size_t)recs_n)) || (e = counters.reserve(8)) || (e = counters64.reserve(2)))
+      return e;
+    hash_cap = hashes, node_cap = nodes_n, rec_cap = recs_n, pool_cap = points;
+    return cudaSuccess;
+  }
+  MapArena arena(const MapCfg &cfg) const {
+    MapArena A{};
+    A.slots = slots.p, A.hash_mask = hash_cap - 1, A.slot_root = slot_root.p, A.slot_cap = slot_cap.p;
+    A.nodes = nodes.p, A.node_cap = node_cap, A.pool = pool.p, A.pool_cap = pool_cap;
+    A.recs = recs.p, A.planes = planes.p, A.rec_node = rec_node.p, A.rec_cap = rec_cap;
+    A.counters = counters.p, A.counters64 = counters64.p, A.cfg = cfg;
+    return A;
+  }
+};
+
+// Loop-control block shared by the kernels of one update. The persistent kernels initialise it from CTA 0; the
+// per-iteration launch path zeroes it with a memset.
+struct CtlBlock {
+  esikf_lio_stats lio_stats;
+  Ctrl ctrl;
+  unsigned char pad[64];
+  esikf_vio_stats vio_stats;
+};
+static_assert(offsetof(CtlBlock, ctrl) == sizeof(esikf_lio_stats) && offsetof(CtlBlock, vio_stats) == sizeof(esikf_lio_stats) + sizeof(Ctrl) + 64 &&
+                  sizeof(CtlBlock) == sizeof(esikf_lio_stats) + sizeof(Ctrl) + 64 + sizeof(esikf_vio_stats),
+              "control block layout [esikf_lio_stats | Ctrl | 64 B pad | esikf_vio_stats]");
 
 #define VIO_PERSIST_SMEM (sizeof(VioSmem) + sizeof(FusedSolveSmem))
 
@@ -101,10 +160,8 @@ struct esikf_ctx {
   double ext_host[12] = {};
 
   // map
-  DevBuf<HashSlot> slots;
+  MapStorage map, map_spare;
   uint32_t hash_mask = 0;
-  DevBuf<esikf_plane> planes;   // the map as uploaded (256-byte records)
-  DevBuf<PlaneRec> recs;        // what the residual kernel reads (144-byte records derived on the device)
   DevBuf<int32_t> patch_ids;
   int n_planes = 0, n_roots = 0;
   double voxel_size = 0.5;
@@ -113,22 +170,12 @@ struct esikf_ctx {
   // device-resident map (esikf_map_device_*): octree nodes, point lists and refits stay on the GPU
   bool dev_map = false;
   esikf_map_cfg map_cfg{};
-  MapArena arena{};
-  DevBuf<int> map_slot_root, map_slot_cap, map_rec_node, map_counters, map_work;
-  DevBuf<unsigned long long> map_counters64;
-  DevBuf<MapNode> map_nodes;
-  DevBuf<double> map_pool, map_pt, map_pt_normal;
+  MapCfg map_kcfg{};           // map_cfg as the map kernels read it
+  DevBuf<int> map_work, map_survivors;
+  DevBuf<double> map_pt, map_pt_normal;
   DevBuf<unsigned int> map_key_in, map_key_out, map_idx_in, map_idx_out;
   DevBuf<MapTouched> map_touched;
   DevBuf<unsigned char> map_sort_tmp;
-  // second arena: esikf_map_device_slide copies the surviving roots into it, then the two change roles
-  DevBuf<HashSlot> slots2;
-  DevBuf<esikf_plane> planes2;
-  DevBuf<PlaneRec> recs2;
-  DevBuf<int> map_slot_root2, map_slot_cap2, map_rec_node2, map_counters2, map_survivors;
-  DevBuf<unsigned long long> map_counters64_2;
-  DevBuf<MapNode> map_nodes2;
-  DevBuf<double> map_pool2;
   int map_pt_n = 0;            // points the normal snapshot / last map step covers
   bool map_normals_valid = false;
   int map_hash_bits = 0;
@@ -147,7 +194,7 @@ struct esikf_ctx {
 
   // shared update state
   DevBuf<double> state_prop;             // [state 386 | prop 386] contiguous: one H2D copy per update
-  struct { double *p; } state, prop;
+  double *state = nullptr, *prop = nullptr;
   DevBuf<double> info, partials, old_state, G;
   // pinned staging ring for the two packed states of an update (slot reuse guarded by an event)
   enum { STAGE_SLOTS = 16 };
@@ -156,11 +203,7 @@ struct esikf_ctx {
   cudaEvent_t stage_ev[STAGE_SLOTS] = {};
   unsigned stage_idx = 0;
   unsigned launch_parity = 0;            // the persistent kernels alternate between two grid-barrier counters
-  DevBuf<unsigned char> ctl_block;  // [esikf_lio_stats | Ctrl | 64 B pad | esikf_vio_stats]; initialised by CTA 0 of the persistent kernels,
-                                    // by a memset on the per-iteration launch path
-  struct { Ctrl *p; } ctrl;
-  struct { esikf_lio_stats *p; } lio_stats;
-  struct { esikf_vio_stats *p; } vio_stats;
+  DevBuf<CtlBlock> ctl;
   int partial_blocks = 0;
 
   // VIO
@@ -182,7 +225,7 @@ struct esikf_ctx {
   DevBuf<int32_t> warp_levels;
   int n_patches = 0;
   // warp producers
-  std::vector<uint8_t *> ref_imgs;
+  std::vector<DevBuf<uint8_t>> ref_imgs;
   DevBuf<const uint8_t *> ref_img_ptrs;
   int ref_w = 0, ref_h = 0;
   DevBuf<int32_t> ref_idx;
@@ -204,8 +247,26 @@ struct esikf_ctx {
   std::vector<cudaEvent_t> ev;      // 3 per slot: before residual, after residual, after solve
   int lio_slots = 0, vio_slots = 0;
   bool lio_timed = false, vio_timed = false;
+  cudaEvent_t prof_ev[2] = {};      // esikf_profile_kernel
   DevBuf<uint8_t> flush;
   DevBuf<double> scratch_state, point_cov_tmp;
+
+  // the device buffers free themselves; this releases what is not a DevBuf (the caller has made `device` current)
+  ~esikf_ctx() {
+    if (stream) cudaStreamSynchronize(stream);
+    if (comm && g_nccl.CommDestroy) g_nccl.CommDestroy(comm);
+    for (size_t r = 0; r < peer_ptrs.size(); r++)
+      if ((int)r != rank && peer_ptrs[r]) cudaIpcCloseMemHandle(peer_ptrs[r]);
+    if (mailbox) cudaFree(mailbox);
+    if (stage) cudaFreeHost(stage);
+    if (stage_ctrl) cudaFreeHost(stage_ctrl);
+    for (cudaEvent_t e : stage_ev)
+      if (e) cudaEventDestroy(e);
+    for (cudaEvent_t e : prof_ev)
+      if (e) cudaEventDestroy(e);
+    for (cudaEvent_t e : ev) cudaEventDestroy(e);
+    if (stream) cudaStreamDestroy(stream);
+  }
 };
 
 static int fail(esikf_ctx *c, int code, const char *fmt, ...) {
@@ -262,26 +323,20 @@ int esikf_create(esikf_ctx **out, int device) {
             cudaMallocHost(&ctx->stage, (size_t)esikf_ctx::STAGE_SLOTS * 2 * S_N * sizeof(double)) == cudaSuccess &&
             cudaMallocHost(&ctx->stage_ctrl, 256) == cudaSuccess &&
             ctx->old_state.reserve(32) == cudaSuccess && ctx->G.reserve(19 * 7) == cudaSuccess &&
-            ctx->ctl_block.reserve(sizeof(esikf_lio_stats) + sizeof(Ctrl) + 64 + sizeof(esikf_vio_stats)) == cudaSuccess && ctx->ext_dev.reserve(12) == cudaSuccess &&
-            ctx->scratch_state.reserve(S_N) == cudaSuccess;
+            ctx->ctl.reserve(1) == cudaSuccess && ctx->ext_dev.reserve(12) == cudaSuccess && ctx->scratch_state.reserve(S_N) == cudaSuccess;
   ctx->partial_blocks = ctx->sm_count < 160 ? ctx->sm_count : 160;  // persistent residual kernels: one CTA per SM
   ok = ok && ctx->partials.reserve((size_t)2 * ctx->partial_blocks * NE_MAX) == cudaSuccess && ctx->stamps.reserve(8 * 72 + 64 + 160) == cudaSuccess &&
        ctx->barrier.reserve(128) == cudaSuccess;
   if (ok) cudaMemsetAsync(ctx->barrier.p, 0, 128 * sizeof(unsigned int), ctx->stream);
   if (ok) {
-    ctx->state.p = ctx->state_prop.p, ctx->prop.p = ctx->state_prop.p + S_N;
+    ctx->state = ctx->state_prop.p, ctx->prop = ctx->state_prop.p + S_N;
     for (int i = 0; i < esikf_ctx::STAGE_SLOTS; i++) ok = ok && cudaEventCreateWithFlags(&ctx->stage_ev[i], cudaEventDisableTiming) == cudaSuccess;
+    for (cudaEvent_t &e : ctx->prof_ev) ok = ok && cudaEventCreate(&e) == cudaSuccess;
   }
-  if (ok) {
-    unsigned char *b = ctx->ctl_block.p;
-    ctx->lio_stats.p = reinterpret_cast<esikf_lio_stats *>(b);
-    ctx->ctrl.p = reinterpret_cast<Ctrl *>(b + sizeof(esikf_lio_stats));
-    ctx->vio_stats.p = reinterpret_cast<esikf_vio_stats *>(b + sizeof(esikf_lio_stats) + sizeof(Ctrl) + 64);
-    cudaMemsetAsync(b, 0, ctx->ctl_block.cap, ctx->stream);
-  }
+  if (ok) cudaMemsetAsync(ctx->ctl.p, 0, sizeof(CtlBlock), ctx->stream);
   cudaDeviceGetAttribute(&ctx->coop_ok, cudaDevAttrCooperativeLaunch, device);
   if (!ok) {
-    esikf_destroy(ctx);
+    delete ctx;
     return ESIKF_ERR_CUDA;
   }
   cudaFuncSetAttribute(lio_residual_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(LioSmem));
@@ -320,33 +375,6 @@ int esikf_create(esikf_ctx **out, int device) {
 void esikf_destroy(esikf_ctx *ctx) {
   if (!ctx) return;
   cudaSetDevice(ctx->device);
-  if (ctx->stream) cudaStreamSynchronize(ctx->stream);
-  if (ctx->comm && g_nccl.CommDestroy) g_nccl.CommDestroy(ctx->comm);
-  for (size_t r = 0; r < ctx->peer_ptrs.size(); r++)
-    if ((int)r != ctx->rank && ctx->peer_ptrs[r]) cudaIpcCloseMemHandle(ctx->peer_ptrs[r]);
-  if (ctx->mailbox) cudaFree(ctx->mailbox);
-  ctx->peer_ptrs_dev.release();
-  ctx->slots.release(), ctx->planes.release(), ctx->recs.release(), ctx->patch_ids.release(), ctx->pts.release(), ctx->pre.release(), ctx->match_plane.release();
-  ctx->normal_plane.release(), ctx->dis.release(), ctx->ext_dev.release(), ctx->state_prop.release();
-  ctx->map_slot_root.release(), ctx->map_slot_cap.release(), ctx->map_rec_node.release(), ctx->map_counters.release(), ctx->map_work.release(), ctx->map_counters64.release();
-  ctx->map_nodes.release(), ctx->map_pool.release(), ctx->map_pt.release(), ctx->map_pt_normal.release(), ctx->map_key_in.release(), ctx->map_key_out.release();
-  ctx->map_idx_in.release(), ctx->map_idx_out.release(), ctx->map_touched.release(), ctx->map_sort_tmp.release();
-  ctx->slots2.release(), ctx->planes2.release(), ctx->recs2.release(), ctx->map_slot_root2.release(), ctx->map_slot_cap2.release(), ctx->map_rec_node2.release();
-  ctx->map_counters2.release(), ctx->map_survivors.release(), ctx->map_counters64_2.release(), ctx->map_nodes2.release(), ctx->map_pool2.release();
-  if (ctx->stage) cudaFreeHost(ctx->stage);
-  if (ctx->stage_ctrl) cudaFreeHost(ctx->stage_ctrl);
-  for (int i = 0; i < esikf_ctx::STAGE_SLOTS; i++)
-    if (ctx->stage_ev[i]) cudaEventDestroy(ctx->stage_ev[i]);
-  ctx->info.release(), ctx->partials.release(), ctx->old_state.release(), ctx->G.release(), ctx->ctl_block.release();
-  ctx->stamps.release(), ctx->barrier.release(), ctx->img.release(), ctx->vis_pos.release(), ctx->inv_expo.release();
-  ctx->warp_patch.release(), ctx->errors.release(), ctx->search_levels.release(), ctx->ref_img_ptrs.release(), ctx->ref_idx.release();
-  ctx->px_ref.release(), ctx->pos_w.release(), ctx->normal_w.release(), ctx->T_ref.release(), ctx->T_cur.release();
-  ctx->warp_out.release(), ctx->warp_levels.release();
-  ctx->inv_ref_px.release(), ctx->inv_ref_f.release(), ctx->inv_ref_R.release(), ctx->inv_ref_pos.release(), ctx->H_sub_inv.release(), ctx->inv_ref_idx.release();
-  ctx->A_cur_ref.release(), ctx->pc_buf.release(), ctx->patch_buf.release(), ctx->flush.release(), ctx->scratch_state.release(), ctx->point_cov_tmp.release();
-  for (uint8_t *p : ctx->ref_imgs) cudaFree(p);
-  for (cudaEvent_t e : ctx->ev) cudaEventDestroy(e);
-  if (ctx->stream) cudaStreamDestroy(ctx->stream);
   delete ctx;
 }
 
@@ -436,13 +464,14 @@ int esikf_map_upload(esikf_ctx *ctx, const int64_t *keys, const int32_t *first, 
     }
     table[s].key = k, table[s].first = (uint32_t)first[r], table[s].count = (uint32_t)count[r];
   }
-  CK(ctx->slots.reserve(cap));
-  CK(ctx->planes.reserve((size_t)n_planes + 1));
-  CK(ctx->recs.reserve((size_t)n_planes + 1));
-  CK(cudaMemcpyAsync(ctx->slots.p, table.data(), cap * sizeof(HashSlot), cudaMemcpyHostToDevice, ctx->stream));
+  MapStorage &M = ctx->map;
+  CK(M.slots.reserve(cap));
+  CK(M.planes.reserve((size_t)n_planes + 1));
+  CK(M.recs.reserve((size_t)n_planes + 1));
+  CK(cudaMemcpyAsync(M.slots.p, table.data(), cap * sizeof(HashSlot), cudaMemcpyHostToDevice, ctx->stream));
   if (n_planes) {
-    CK(cudaMemcpyAsync(ctx->planes.p, planes, (size_t)n_planes * sizeof(esikf_plane), cudaMemcpyHostToDevice, ctx->stream));
-    plane_compact_kernel<<<(n_planes + 127) / 128, 128, 0, ctx->stream>>>(ctx->planes.p, nullptr, n_planes, ctx->recs.p);
+    CK(cudaMemcpyAsync(M.planes.p, planes, (size_t)n_planes * sizeof(esikf_plane), cudaMemcpyHostToDevice, ctx->stream));
+    plane_compact_kernel<<<(n_planes + 127) / 128, 128, 0, ctx->stream>>>(M.planes.p, nullptr, n_planes, M.recs.p);
     ctx->launches++;
   }
   CK(cudaStreamSynchronize(ctx->stream));
@@ -464,13 +493,12 @@ int esikf_map_patch(esikf_ctx *ctx, const int32_t *plane_ids, const esikf_plane 
   for (int i = 0; i < n;) {
     int j = i + 1;
     while (j < n && plane_ids[j] == plane_ids[j - 1] + 1) j++;  // a run of consecutive ids travels as one copy
-    CK(cudaMemcpyAsync(ctx->planes.p + plane_ids[i], planes + i, (size_t)(j - i) * sizeof(esikf_plane), cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(ctx->map.planes.p + plane_ids[i], planes + i, (size_t)(j - i) * sizeof(esikf_plane), cudaMemcpyHostToDevice, ctx->stream));
     i = j;
   }
   if (n > 0) {
-    CK(ctx->patch_ids.reserve(n));
-    CK(cudaMemcpyAsync(ctx->patch_ids.p, plane_ids, (size_t)n * sizeof(int32_t), cudaMemcpyHostToDevice, ctx->stream));
-    plane_compact_kernel<<<(n + 127) / 128, 128, 0, ctx->stream>>>(ctx->planes.p, ctx->patch_ids.p, n, ctx->recs.p);
+    CK(ctx->patch_ids.upload(plane_ids, n, n, ctx->stream));
+    plane_compact_kernel<<<(n + 127) / 128, 128, 0, ctx->stream>>>(ctx->map.planes.p, ctx->patch_ids.p, n, ctx->map.recs.p);
     ctx->launches++;
   }
   CK(cudaStreamSynchronize(ctx->stream));
@@ -481,14 +509,14 @@ int esikf_map_patch(esikf_ctx *ctx, const int32_t *plane_ids, const esikf_plane 
 static int map_check_errors(esikf_ctx *ctx, const char *what) {
   int c[4];
   unsigned long long pool_used = 0;
-  CK(cudaMemcpyAsync(c, ctx->map_counters.p, sizeof(c), cudaMemcpyDeviceToHost, ctx->stream));
-  CK(cudaMemcpyAsync(&pool_used, ctx->map_counters64.p, sizeof(pool_used), cudaMemcpyDeviceToHost, ctx->stream));
+  CK(cudaMemcpyAsync(c, ctx->map.counters.p, sizeof(c), cudaMemcpyDeviceToHost, ctx->stream));
+  CK(cudaMemcpyAsync(&pool_used, ctx->map.counters64.p, sizeof(pool_used), cudaMemcpyDeviceToHost, ctx->stream));
   int work[2];
   CK(cudaMemcpyAsync(work, ctx->map_work.p, sizeof(work), cudaMemcpyDeviceToHost, ctx->stream));
   CK(cudaStreamSynchronize(ctx->stream));
   ctx->map_last.nodes = c[0], ctx->map_last.records = c[1], ctx->map_last.errors = c[2], ctx->map_last.roots = c[3];
   ctx->map_last.pool_points = (int64_t)pool_used, ctx->map_last.touched_roots = work[0];
-  ctx->n_planes = c[1] < (int)ctx->arena.rec_cap ? c[1] : (int)ctx->arena.rec_cap;
+  ctx->n_planes = c[1] < ctx->map.rec_cap ? c[1] : ctx->map.rec_cap;
   ctx->n_roots = c[3];
   if (c[2]) {
     ctx->have_map = false;  // the map is not trustworthy any more: the next lio_run must not use it
@@ -513,26 +541,13 @@ int esikf_map_device_init(esikf_ctx *ctx, const esikf_map_cfg *cfg) {
   const int64_t rec_cap = cfg->record_capacity > 0 ? cfg->record_capacity : 4 * roots;
   const int64_t pool_cap = cfg->point_capacity > 0 ? cfg->point_capacity : 64 * roots;
   if (node_cap > 0x7fffffff || rec_cap > 0x7fffffff || pool_cap > 0x7fffffff) return fail(ctx, ESIKF_ERR_ARG, "map_device_init: capacity above 2^31");
-  CK(ctx->slots.reserve(cap));
-  CK(ctx->map_slot_root.reserve(cap));
-  CK(ctx->map_slot_cap.reserve(cap));
-  CK(ctx->map_nodes.reserve((size_t)node_cap));
-  CK(ctx->map_pool.reserve((size_t)pool_cap * MAP_PT_D));
-  CK(ctx->recs.reserve((size_t)rec_cap));
-  CK(ctx->planes.reserve((size_t)rec_cap));
-  CK(ctx->map_rec_node.reserve((size_t)rec_cap));
-  CK(ctx->map_counters.reserve(8));
-  CK(ctx->map_counters64.reserve(2));
+  CK(ctx->map.reserve(cap, (int)node_cap, (int)rec_cap, pool_cap));
   CK(ctx->map_work.reserve(4));
-  MapArena &A = ctx->arena;
-  A.slots = ctx->slots.p, A.hash_mask = cap - 1, A.slot_root = ctx->map_slot_root.p, A.slot_cap = ctx->map_slot_cap.p;
-  A.nodes = ctx->map_nodes.p, A.node_cap = (int)node_cap, A.pool = ctx->map_pool.p, A.pool_cap = pool_cap;
-  A.recs = ctx->recs.p, A.planes = ctx->planes.p, A.rec_node = ctx->map_rec_node.p, A.rec_cap = (int)rec_cap;
-  A.counters = ctx->map_counters.p, A.counters64 = ctx->map_counters64.p;
-  A.cfg.voxel_size = (float)cfg->voxel_size, A.cfg.planer_threshold = (float)cfg->min_eigen_value;
-  A.cfg.max_layer = cfg->max_layer, A.cfg.max_points_num = cfg->max_points_num;
-  for (int k = 0; k < MAP_MAX_LAYERS; k++) A.cfg.layer_init_num[k] = cfg->layer_init_num[k <= cfg->max_layer ? k : cfg->max_layer];
-  map_reset_kernel<<<(cap + 255) / 256, 256, 0, ctx->stream>>>(A);
+  MapCfg &K = ctx->map_kcfg;
+  K.voxel_size = (float)cfg->voxel_size, K.planer_threshold = (float)cfg->min_eigen_value;
+  K.max_layer = cfg->max_layer, K.max_points_num = cfg->max_points_num;
+  for (int k = 0; k < MAP_MAX_LAYERS; k++) K.layer_init_num[k] = cfg->layer_init_num[k <= cfg->max_layer ? k : cfg->max_layer];
+  map_reset_kernel<<<(cap + 255) / 256, 256, 0, ctx->stream>>>(ctx->map.arena(K));
   CK(cudaMemsetAsync(ctx->map_work.p, 0, 4 * sizeof(int), ctx->stream));
   CK(cudaStreamSynchronize(ctx->stream));
   ctx->launches++;
@@ -550,7 +565,7 @@ int esikf_map_device_init(esikf_ctx *ctx, const esikf_map_cfg *cfg) {
 // sort by slot, list the touched roots, replay them
 static int map_apply_points(esikf_ctx *ctx, int n, bool build) {
   cudaStream_t st = ctx->stream;
-  const unsigned int invalid = ctx->arena.hash_mask + 1u;
+  const unsigned int invalid = ctx->map.hash_cap;
   size_t tmp_bytes = 0;
   cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, ctx->map_key_in.p, ctx->map_key_out.p, ctx->map_idx_in.p, ctx->map_idx_out.p, n, 0, ctx->map_hash_bits + 1, st);
   CK(ctx->map_sort_tmp.reserve(tmp_bytes + 16));
@@ -558,7 +573,7 @@ static int map_apply_points(esikf_ctx *ctx, int n, bool build) {
                                      ctx->map_hash_bits + 1, st));
   CK(cudaMemsetAsync(ctx->map_work.p, 0, 2 * sizeof(int), st));
   map_heads_kernel<<<(n + 255) / 256, 256, 0, st>>>(ctx->map_key_out.p, n, invalid, ctx->map_touched.p, ctx->map_work.p);
-  map_replay_kernel<<<ctx->sm_count * 4, 128, 0, st>>>(ctx->arena, ctx->map_touched.p, ctx->map_work.p, ctx->map_idx_out.p, ctx->map_pt.p, build ? 1 : 0);
+  map_replay_kernel<<<ctx->sm_count * 4, 128, 0, st>>>(ctx->map.arena(ctx->map_kcfg), ctx->map_touched.p, ctx->map_work.p, ctx->map_idx_out.p, ctx->map_pt.p, build ? 1 : 0);
   ctx->launches += 4;
   CK(cudaGetLastError());
   return map_check_errors(ctx, build ? "map_device_build" : "map_device_update");
@@ -587,10 +602,9 @@ static int map_from_scan(esikf_ctx *ctx, const double *state, bool build) {
   int rc = map_reserve_tick(ctx, n);
   if (rc) return rc;
   cudaStream_t st = ctx->stream;
-  const double *dev_state = ctx->state.p;  // the posterior the last update left on the device
+  const double *dev_state = ctx->state;  // the posterior the last update left on the device
   if (state) {
-    CK(ctx->scratch_state.reserve(S_N));
-    CK(cudaMemcpyAsync(ctx->scratch_state.p, state, S_N * sizeof(double), cudaMemcpyHostToDevice, st));
+    CK(ctx->scratch_state.upload(state, S_N, S_N, st));
     dev_state = ctx->scratch_state.p;
   }
   MapPointArgs a;
@@ -598,9 +612,9 @@ static int map_from_scan(esikf_ctx *ctx, const double *state, bool build) {
   a.pts = ctx->pts.p, a.pre = ctx->pre.p, a.pre_stride = ctx->pre_stride, a.n = n, a.state = dev_state;
   memcpy(a.extR, ctx->ext.extR, 72), memcpy(a.extT, ctx->ext.extT, 24);
   a.build = build ? 1 : 0, a.dept_err = (float)ctx->map_cfg.dept_err, a.beam_err = (float)ctx->map_cfg.beam_err;
-  a.match_plane = build ? nullptr : ctx->normal_plane.p, a.recs = ctx->recs.p, a.pt_normal = ctx->map_pt_normal.p;
-  a.pt = ctx->map_pt.p, a.pt_slot = ctx->map_key_in.p, a.pt_idx = ctx->map_idx_in.p, a.invalid_slot = ctx->arena.hash_mask + 1u;
-  map_points_kernel<<<(n + 255) / 256, 256, 0, st>>>(ctx->arena, a);
+  a.match_plane = build ? nullptr : ctx->normal_plane.p, a.recs = ctx->map.recs.p, a.pt_normal = ctx->map_pt_normal.p;
+  a.pt = ctx->map_pt.p, a.pt_slot = ctx->map_key_in.p, a.pt_idx = ctx->map_idx_in.p, a.invalid_slot = ctx->map.hash_cap;
+  map_points_kernel<<<(n + 255) / 256, 256, 0, st>>>(ctx->map.arena(ctx->map_kcfg), a);
   ctx->map_pt_n = n, ctx->map_normals_valid = !build;
   return map_apply_points(ctx, n, build);
 }
@@ -622,7 +636,7 @@ int esikf_map_device_update_points(esikf_ctx *ctx, const double *point_w, const 
   // [n][12] = point_w | var: two strided copies
   CK(cudaMemcpy2DAsync(ctx->map_pt.p, MAP_PT_D * sizeof(double), point_w, 3 * sizeof(double), 3 * sizeof(double), n, cudaMemcpyHostToDevice, st));
   CK(cudaMemcpy2DAsync(ctx->map_pt.p + 3, MAP_PT_D * sizeof(double), var, 9 * sizeof(double), 9 * sizeof(double), n, cudaMemcpyHostToDevice, st));
-  map_keys_kernel<<<(n + 255) / 256, 256, 0, st>>>(ctx->arena, ctx->map_pt.p, n, ctx->map_key_in.p, ctx->map_idx_in.p, ctx->arena.hash_mask + 1u);
+  map_keys_kernel<<<(n + 255) / 256, 256, 0, st>>>(ctx->map.arena(ctx->map_kcfg), ctx->map_pt.p, n, ctx->map_key_in.p, ctx->map_idx_in.p, ctx->map.hash_cap);
   ctx->launches++;
   ctx->map_normals_valid = false;
   return map_apply_points(ctx, n, false);
@@ -634,22 +648,11 @@ int esikf_map_device_slide(esikf_ctx *ctx, const int64_t key_min[3], const int64
   if (!ctx->dev_map) return fail(ctx, ESIKF_ERR_STATE, "map_device_slide before esikf_map_device_init");
   CK(cudaSetDevice(ctx->device));
   cudaStream_t st = ctx->stream;
-  const MapArena S = ctx->arena;
-  const unsigned cap = S.hash_mask + 1u;
-  CK(ctx->slots2.reserve(cap));
-  CK(ctx->map_slot_root2.reserve(cap));
-  CK(ctx->map_slot_cap2.reserve(cap));
-  CK(ctx->map_nodes2.reserve((size_t)S.node_cap));
-  CK(ctx->map_pool2.reserve((size_t)S.pool_cap * MAP_PT_D));
-  CK(ctx->recs2.reserve((size_t)S.rec_cap));
-  CK(ctx->planes2.reserve((size_t)S.rec_cap));
-  CK(ctx->map_rec_node2.reserve((size_t)S.rec_cap));
-  CK(ctx->map_counters2.reserve(8));
-  CK(ctx->map_counters64_2.reserve(2));
+  const MapStorage &M = ctx->map;
+  const unsigned cap = M.hash_cap;
+  CK(ctx->map_spare.reserve(cap, M.node_cap, M.rec_cap, M.pool_cap));
   CK(ctx->map_survivors.reserve((size_t)(ctx->map_last.roots > 0 ? ctx->map_last.roots : 1) + 1));
-  MapArena D = S;
-  D.slots = ctx->slots2.p, D.slot_root = ctx->map_slot_root2.p, D.slot_cap = ctx->map_slot_cap2.p, D.nodes = ctx->map_nodes2.p, D.pool = ctx->map_pool2.p;
-  D.recs = ctx->recs2.p, D.planes = ctx->planes2.p, D.rec_node = ctx->map_rec_node2.p, D.counters = ctx->map_counters2.p, D.counters64 = ctx->map_counters64_2.p;
+  const MapArena S = M.arena(ctx->map_kcfg), D = ctx->map_spare.arena(ctx->map_kcfg);
   const long long big = 1ll << 40;
   const long long lo[3] = {key_min ? key_min[0] : -big, key_min ? key_min[1] : -big, key_min ? key_min[2] : -big};
   const long long hi[3] = {key_max ? key_max[0] : big, key_max ? key_max[1] : big, key_max ? key_max[2] : big};
@@ -660,10 +663,7 @@ int esikf_map_device_slide(esikf_ctx *ctx, const int64_t key_min[3], const int64
   ctx->launches += 3;
   CK(cudaGetLastError());
   // the fresh arena becomes the map (also when the copy reports an error: the status says so and the map is invalidated)
-  std::swap(ctx->slots, ctx->slots2), std::swap(ctx->map_slot_root, ctx->map_slot_root2), std::swap(ctx->map_slot_cap, ctx->map_slot_cap2);
-  std::swap(ctx->map_nodes, ctx->map_nodes2), std::swap(ctx->map_pool, ctx->map_pool2), std::swap(ctx->recs, ctx->recs2), std::swap(ctx->planes, ctx->planes2);
-  std::swap(ctx->map_rec_node, ctx->map_rec_node2), std::swap(ctx->map_counters, ctx->map_counters2), std::swap(ctx->map_counters64, ctx->map_counters64_2);
-  ctx->arena = D;
+  std::swap(ctx->map, ctx->map_spare);
   ctx->map_normals_valid = false;  // record positions of the last update are gone
   return map_check_errors(ctx, "map_device_slide");
 }
@@ -694,8 +694,8 @@ int esikf_map_device_download(esikf_ctx *ctx, int64_t *keys, int32_t *first, int
     CK(d_count.reserve(roots_cap));
     CK(d_planes.reserve(planes_cap > 0 ? planes_cap : 1));
   }
-  const unsigned cap = ctx->arena.hash_mask + 1u;
-  map_download_kernel<<<(cap + 255) / 256, 256, 0, st>>>(ctx->arena, fill ? d_keys.p : nullptr, d_first.p, d_count.p, d_planes.p, fill ? roots_cap : 0, fill ? planes_cap : 0, d_out.p);
+  const unsigned cap = ctx->map.hash_cap;
+  map_download_kernel<<<(cap + 255) / 256, 256, 0, st>>>(ctx->map.arena(ctx->map_kcfg), fill ? d_keys.p : nullptr, d_first.p, d_count.p, d_planes.p, fill ? roots_cap : 0, fill ? planes_cap : 0, d_out.p);
   ctx->launches++;
   int out[2];
   CK(cudaMemcpyAsync(out, d_out.p, sizeof(out), cudaMemcpyDeviceToHost, st));
@@ -712,7 +712,6 @@ int esikf_map_device_download(esikf_ctx *ctx, int64_t *keys, int32_t *first, int
       if (out[1]) CK(cudaMemcpy(planes, d_planes.p, (size_t)out[1] * sizeof(esikf_plane), cudaMemcpyDeviceToHost));
     }
   }
-  d_keys.release(), d_first.release(), d_count.release(), d_planes.release(), d_out.release();
   return rc;
 }
 
@@ -733,7 +732,7 @@ int esikf_lio_fetch_normals(esikf_ctx *ctx, double *normals) {
   if (n == 0) return ESIKF_OK;
   if (!(ctx->dev_map && ctx->map_normals_valid && ctx->map_pt_n == n)) {
     CK(ctx->map_pt_normal.reserve((size_t)n * 3 + 4));
-    gather_normals_kernel<<<(n + 255) / 256, 256, 0, ctx->stream>>>(ctx->normal_plane.p, ctx->recs.p, n, ctx->map_pt_normal.p);
+    gather_normals_kernel<<<(n + 255) / 256, 256, 0, ctx->stream>>>(ctx->normal_plane.p, ctx->map.recs.p, n, ctx->map_pt_normal.p);
     ctx->launches++;
   }
   CK(cudaMemcpyAsync(normals, ctx->map_pt_normal.p, (size_t)n * 3 * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
@@ -745,26 +744,25 @@ int esikf_lio_fetch_normals(esikf_ctx *ctx, double *normals) {
 int esikf_lio_set_scan(esikf_ctx *ctx, const float *pts_xyz, int32_t n) {
   if (!ctx || n < 0 || (n > 0 && !pts_xyz)) return fail(ctx, ESIKF_ERR_ARG, "lio_set_scan: bad argument");
   CK(cudaSetDevice(ctx->device));
-  CK(ctx->pts.reserve((size_t)n * 3 + 4));
   ctx->pre_stride = (n + 31) & ~31;
   CK(ctx->pre.reserve((size_t)ctx->pre_stride * 9 + 16));
   CK(ctx->match_plane.reserve(n + 1));
   CK(ctx->normal_plane.reserve(n + 1));
   CK(ctx->dis.reserve(n + 1));
-  if (n) CK(cudaMemcpyAsync(ctx->pts.p, pts_xyz, (size_t)n * 3 * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
+  CK(ctx->pts.upload(pts_xyz, (size_t)n * 3, (size_t)n * 3 + 4, ctx->stream));
   ctx->n_pts = n;
   ctx->scan_fresh = true;
   return ESIKF_OK;
 }
 
-static int lio_fill_args(esikf_ctx *ctx, LioKernelArgs &ka, double *state_ptr) {
+static void lio_fill_args(esikf_ctx *ctx, LioKernelArgs &ka, double *state_ptr) {
   memset(&ka, 0, sizeof(ka));
   ka.pts = ctx->pts.p, ka.pre = ctx->pre.p;
   ka.pre_stride = ctx->pre_stride;
   ka.partial_stride = ctx->partial_blocks;
   shard_of(ctx->n_pts, ctx->rank, ctx->nranks, ka.begin, ka.count);
-  ka.state = state_ptr, ka.prop = ctx->prop.p;
-  ka.slots = ctx->slots.p, ka.hash_mask = ctx->hash_mask, ka.recs = ctx->recs.p;
+  ka.state = state_ptr, ka.prop = ctx->prop;
+  ka.slots = ctx->map.slots.p, ka.hash_mask = ctx->hash_mask, ka.recs = ctx->map.recs.p;
   ka.stage_mode = (ctx->tuning & ESIKF_TUNE_STAGE_LDG) ? 1 : 0;
   memcpy(ka.extR, ctx->ext.extR, sizeof(ka.extR));
   memcpy(ka.extT, ctx->ext.extT, sizeof(ka.extT));
@@ -777,8 +775,15 @@ static int lio_fill_args(esikf_ctx *ctx, LioKernelArgs &ka, double *state_ptr) {
   ka.voxel_size_f = (float)ctx->lio_cfg.voxel_size;
   ka.sigma_num = ctx->lio_cfg.sigma_num;
   ka.match_plane = ctx->match_plane.p, ka.normal_plane = ctx->normal_plane.p, ka.dis_to_plane = ctx->dis.p;
-  ka.partials = ctx->partials.p, ka.info = ctx->info.p, ka.ctrl = ctx->ctrl.p;
-  return 0;
+  ka.partials = ctx->partials.p, ka.info = ctx->info.p, ka.ctrl = &ctx->ctl.p->ctrl;
+}
+// the SolveArgs fields every solve launch sets; the LIO / VIO specific ones are the caller's
+static SolveArgs solve_args(esikf_ctx *ctx, double *state_ptr, int max_iterations) {
+  SolveArgs sa;
+  memset(&sa, 0, sizeof(sa));
+  sa.state = state_ptr, sa.prop = ctx->prop, sa.info = ctx->info.p, sa.ctrl = &ctx->ctl.p->ctrl;
+  sa.max_iterations = max_iterations, sa.solve_mode = ctx->solve_mode;
+  return sa;
 }
 static int lio_grid(const esikf_ctx *ctx, int count) {
   int chunks = (count + 31) / 32;  // whole warps are dealt to the CTAs: every SM takes part as soon as there is a warp for it
@@ -796,12 +801,32 @@ static int upload_states(esikf_ctx *ctx, const double *state_in, const double *s
   CK(cudaEventRecord(ctx->stage_ev[slot], ctx->stream));
   return ESIKF_OK;
 }
-static PeerArgs peer_args(esikf_ctx *ctx) {
-  PeerArgs p;
-  p.mbox = ctx->p2p ? ctx->peer_ptrs_dev.p : nullptr;
-  p.seq = ctx->peer_seq_dev;
-  p.rank = ctx->rank, p.nranks = ctx->p2p ? ctx->nranks : 1;
-  return p;
+// Whether an update runs as one persistent cooperative kernel (`coop`: co-resident CTAs per SM of that kernel).
+static bool persistent_ok(const esikf_ctx *ctx, int coop) {
+  return ctx->loop_mode >= 1 && (ctx->nranks == 1 || ctx->p2p) && ctx->coop_ok && coop > 0 && !ctx->timing;
+}
+// One cooperative launch of a persistent update kernel. `fn_solo` / `fn_peers` are its instantiations without and with
+// the NVLink peer exchange; their parameters are (ka, sa, barrier, barrier_next, stamps, parity_stride, peer[, inv, tma]).
+// The kernel's phase stamps go to `stamp_words` words at `stamps + stamp_off`.
+static int launch_persistent(esikf_ctx *ctx, const char *name, const void *fn_solo, const void *fn_peers, int grid, int threads, size_t smem,
+                             size_t stamp_off, size_t stamp_words, void *ka, SolveArgs *sa, void *inv, void *tma, bool &timed) {
+  const unsigned par = ctx->launch_parity & 1;
+  unsigned int *bar = ctx->barrier.p + 64 * par, *bar_next = ctx->barrier.p + 64 * (par ^ 1);  // this launch's barrier / the next launch's (zeroed by the kernel)
+  unsigned long long *stamps = ctx->want_stamps ? ctx->stamps.p + stamp_off : nullptr;
+  if (stamps) CK(cudaMemsetAsync(stamps, 0, stamp_words * sizeof(unsigned long long), ctx->stream));
+  size_t parity_stride = (size_t)ctx->partial_blocks * NE_MAX;
+  PeerArgs peer;
+  peer.mbox = ctx->p2p ? ctx->peer_ptrs_dev.p : nullptr;
+  peer.seq = ctx->peer_seq_dev;
+  peer.rank = ctx->rank, peer.nranks = ctx->p2p ? ctx->nranks : 1;
+  void *kargs[] = {ka, (void *)sa, (void *)&bar, (void *)&bar_next, (void *)&stamps, (void *)&parity_stride, (void *)&peer, inv, tma};
+  const void *fn = (ctx->p2p && ctx->nranks > 1) ? fn_peers : fn_solo;
+  cudaError_t le = cudaLaunchCooperativeKernel(fn, dim3(grid), dim3(threads), kargs, smem, ctx->stream);
+  if (le != cudaSuccess) return fail(ctx, ESIKF_ERR_CUDA, "cooperative launch of %s failed: %s", name, cudaGetErrorString(le));
+  ctx->launch_parity++;  // only a launch that happened consumes its barrier counter (the kernel zeroes the other one)
+  ctx->launches += 1;
+  timed = false;
+  return ESIKF_OK;
 }
 static int allreduce_info(esikf_ctx *ctx) {
   if (ctx->nranks <= 1) return ESIKF_OK;
@@ -824,9 +849,9 @@ int esikf_lio_run(esikf_ctx *ctx, const double *state_in, const double *state_pr
     int rc = upload_states(ctx, state_in, state_prop);
     if (rc) return rc;
   }
-  const bool fused_lio = ctx->loop_mode >= 1 && (ctx->nranks == 1 || ctx->p2p) && ctx->coop_ok && ctx->coop_lio > 0 && !ctx->timing;
+  const bool fused_lio = persistent_ok(ctx, ctx->coop_lio);
   // the persistent kernel initialises its own loop control / stats / barrier; the per-iteration path needs them zeroed
-  if (!fused_lio) CK(cudaMemsetAsync(ctx->lio_stats.p, 0, sizeof(esikf_lio_stats) + sizeof(Ctrl) + 64, st));
+  if (!fused_lio) CK(cudaMemsetAsync(&ctx->ctl.p->lio_stats, 0, offsetof(CtlBlock, vio_stats), st));
   const int n = ctx->n_pts;
   if (ctx->scan_fresh) {
     if (n > 0) {
@@ -836,28 +861,13 @@ int esikf_lio_run(esikf_ctx *ctx, const double *state_in, const double *state_pr
     ctx->scan_fresh = false;
   }
   LioKernelArgs ka;
-  lio_fill_args(ctx, ka, ctx->state.p);
-  SolveArgs sa;
-  memset(&sa, 0, sizeof(sa));
-  sa.state = ctx->state.p, sa.prop = ctx->prop.p, sa.info = ctx->info.p, sa.ctrl = ctx->ctrl.p;
-  sa.max_iterations = cfg->max_iterations, sa.solve_mode = ctx->solve_mode, sa.lio_stats = ctx->lio_stats.p;
+  lio_fill_args(ctx, ka, ctx->state);
+  SolveArgs sa = solve_args(ctx, ctx->state, cfg->max_iterations);
+  sa.lio_stats = &ctx->ctl.p->lio_stats;
   const int grid = lio_grid(ctx, ka.count);
-  if (fused_lio) {
-    const unsigned par = ctx->launch_parity & 1;
-    unsigned int *bar = ctx->barrier.p + 64 * par, *bar_next = ctx->barrier.p + 64 * (par ^ 1);  // this launch's barrier / the next launch's (zeroed by the kernel)
-    unsigned long long *stamps = ctx->want_stamps ? ctx->stamps.p : nullptr;
-    if (stamps) CK(cudaMemsetAsync(stamps, 0, 64 * sizeof(unsigned long long), st));
-    size_t parity_stride = (size_t)ctx->partial_blocks * NE_MAX;
-    PeerArgs peer = peer_args(ctx);
-    void *kargs[] = {(void *)&ka, (void *)&sa, (void *)&bar, (void *)&bar_next, (void *)&stamps, (void *)&parity_stride, (void *)&peer};
-    const void *fn = (ctx->p2p && ctx->nranks > 1) ? (const void *)lio_update_kernel<true> : (const void *)lio_update_kernel<false>;
-    cudaError_t le = cudaLaunchCooperativeKernel(fn, dim3(grid), dim3(LIO_THREADS), kargs, sizeof(LioSmem), st);
-    if (le != cudaSuccess) return fail(ctx, ESIKF_ERR_CUDA, "cooperative launch of lio_update_kernel failed: %s", cudaGetErrorString(le));
-    ctx->launch_parity++;  // only a launch that happened consumes its barrier counter (the kernel zeroes the other one)
-    ctx->launches += 1;
-    ctx->lio_timed = false;
-    return ESIKF_OK;
-  }
+  if (fused_lio)
+    return launch_persistent(ctx, "lio_update_kernel", (const void *)lio_update_kernel<false>, (const void *)lio_update_kernel<true>, grid, LIO_THREADS,
+                             sizeof(LioSmem), 0, 64, &ka, &sa, nullptr, nullptr, ctx->lio_timed);
   ctx->lio_timed = ctx->timing;
   ctx->lio_slots = cfg->max_iterations;
   for (int it = 0; it < cfg->max_iterations; it++) {
@@ -880,10 +890,10 @@ int esikf_lio_run(esikf_ctx *ctx, const double *state_in, const double *state_pr
 // (Ctrl::comm_error, sticky on the device) into ESIKF_ERR_COMM once.
 static int finish_fetch(esikf_ctx *ctx) {
   Ctrl *h = reinterpret_cast<Ctrl *>(ctx->stage_ctrl);
-  CK(cudaMemcpyAsync(h, ctx->ctrl.p, sizeof(Ctrl), cudaMemcpyDeviceToHost, ctx->stream));
+  CK(cudaMemcpyAsync(h, &ctx->ctl.p->ctrl, sizeof(Ctrl), cudaMemcpyDeviceToHost, ctx->stream));
   CK(cudaStreamSynchronize(ctx->stream));
   if (h->comm_error) {
-    cudaMemsetAsync(&ctx->ctrl.p->comm_error, 0, sizeof(int), ctx->stream);
+    cudaMemsetAsync(&ctx->ctl.p->ctrl.comm_error, 0, sizeof(int), ctx->stream);
     return fail(ctx, ESIKF_ERR_COMM, "a bounded in-kernel wait expired (grid barrier or peer mailbox): a rank did not take part in the update");
   }
   return ESIKF_OK;
@@ -894,8 +904,8 @@ int esikf_lio_fetch(esikf_ctx *ctx, double *state_out, esikf_lio_stats *stats, i
   CK(cudaSetDevice(ctx->device));
   cudaStream_t st = ctx->stream;
   const size_t n = (size_t)ctx->n_pts;
-  if (state_out) CK(cudaMemcpyAsync(state_out, ctx->state.p, S_N * sizeof(double), cudaMemcpyDeviceToHost, st));
-  if (stats) CK(cudaMemcpyAsync(stats, ctx->lio_stats.p, sizeof(esikf_lio_stats), cudaMemcpyDeviceToHost, st));
+  if (state_out) CK(cudaMemcpyAsync(state_out, ctx->state, S_N * sizeof(double), cudaMemcpyDeviceToHost, st));
+  if (stats) CK(cudaMemcpyAsync(stats, &ctx->ctl.p->lio_stats, sizeof(esikf_lio_stats), cudaMemcpyDeviceToHost, st));
   if (match_plane && n) CK(cudaMemcpyAsync(match_plane, ctx->match_plane.p, n * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
   if (normal_plane && n) CK(cudaMemcpyAsync(normal_plane, ctx->normal_plane.p, n * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
   if (dis_to_plane && n) CK(cudaMemcpyAsync(dis_to_plane, ctx->dis.p, n * sizeof(float), cudaMemcpyDeviceToHost, st));
@@ -959,33 +969,39 @@ int esikf_vio_set_image(esikf_ctx *ctx, const uint8_t *img, int32_t width, int32
   if (!ctx->have_cam) return fail(ctx, ESIKF_ERR_STATE, "vio_set_image before vio_set_camera");
   if (width != ctx->cam.width || height != ctx->cam.height) return fail(ctx, ESIKF_ERR_ARG, "vio_set_image: image is %dx%d, camera %dx%d", width, height, ctx->cam.width, ctx->cam.height);
   CK(cudaSetDevice(ctx->device));
-  CK(ctx->img.reserve((size_t)width * height + 64));
-  CK(cudaMemcpyAsync(ctx->img.p, img, (size_t)width * height, cudaMemcpyHostToDevice, ctx->stream));
+  CK(ctx->img.upload(img, (size_t)width * height, (size_t)width * height + 64, ctx->stream));
   ctx->img_w = width, ctx->img_h = height;
+  return ESIKF_OK;
+}
+
+// The kernels shift by the tap stride 1 << (level + search_level) and index the per-stride tensor maps with it: search
+// levels must lie in [0, 8]. `name_patch` adds the patch number to the message.
+static int check_search_levels(esikf_ctx *ctx, const char *what, const int32_t *levels, int n, bool name_patch) {
+  for (int i = 0; i < n; i++)
+    if (levels[i] < 0 || levels[i] > 8)
+      return name_patch ? fail(ctx, ESIKF_ERR_ARG, "%s: search level %d of patch %d", what, levels[i], i) : fail(ctx, ESIKF_ERR_ARG, "%s: search level %d", what, levels[i]);
+  return ESIKF_OK;
+}
+static int check_ref_indices(esikf_ctx *ctx, const char *what, const int32_t *ref_img_index, int n) {
+  for (int i = 0; i < n; i++)
+    if (ref_img_index[i] < 0 || ref_img_index[i] >= (int)ctx->ref_imgs.size()) return fail(ctx, ESIKF_ERR_ARG, "%s: ref image index %d", what, ref_img_index[i]);
   return ESIKF_OK;
 }
 
 int esikf_vio_set_patches(esikf_ctx *ctx, const double *pos, const float *warp_patch, const int32_t *search_levels, const double *inv_expo_list, int32_t n) {
   if (!ctx || n < 0 || (n > 0 && (!pos || !warp_patch || !search_levels || !inv_expo_list))) return fail(ctx, ESIKF_ERR_ARG, "vio_set_patches: bad argument");
   if (!ctx->have_cam) return fail(ctx, ESIKF_ERR_STATE, "vio_set_patches before vio_set_camera");
-  // the kernels shift by the tap stride 1 << (level + search_level) and index the per-stride tensor maps with it: same range
-  // as warp_affine, checked before anything is uploaded so the installed patches stay as they were
-  for (int i = 0; i < n; i++)
-    if (search_levels[i] < 0 || search_levels[i] > 8) return fail(ctx, ESIKF_ERR_ARG, "vio_set_patches: search level %d of patch %d", search_levels[i], i);
+  // checked before anything is uploaded so the installed patches stay as they were
+  int rc = check_search_levels(ctx, "vio_set_patches", search_levels, n, true);
+  if (rc) return rc;
   CK(cudaSetDevice(ctx->device));
-  const int L = ctx->vio_cfg.patch_pyrimid_level;
-  CK(ctx->vis_pos.reserve((size_t)n * 3 + 4));
-  CK(ctx->warp_patch.reserve((size_t)n * 64 * L + 64));
-  CK(ctx->search_levels.reserve(n + 1));
-  CK(ctx->inv_expo.reserve(n + 1));
-  CK(ctx->errors.reserve(n + 1));
+  const size_t L = ctx->vio_cfg.patch_pyrimid_level;
   cudaStream_t st = ctx->stream;
-  if (n) {
-    CK(cudaMemcpyAsync(ctx->vis_pos.p, pos, (size_t)n * 3 * sizeof(double), cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(ctx->warp_patch.p, warp_patch, (size_t)n * 64 * L * sizeof(float), cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(ctx->search_levels.p, search_levels, (size_t)n * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(ctx->inv_expo.p, inv_expo_list, (size_t)n * sizeof(double), cudaMemcpyHostToDevice, st));
-  }
+  CK(ctx->vis_pos.upload(pos, (size_t)n * 3, (size_t)n * 3 + 4, st));
+  CK(ctx->warp_patch.upload(warp_patch, n * 64 * L, n * 64 * L + 64, st));
+  CK(ctx->search_levels.upload(search_levels, n, n + 1, st));
+  CK(ctx->inv_expo.upload(inv_expo_list, n, n + 1, st));
+  CK(ctx->errors.reserve(n + 1));
   ctx->n_patches = n;
   return ESIKF_OK;
 }
@@ -1021,7 +1037,7 @@ static void vio_fill_args(esikf_ctx *ctx, VioKernelArgs &ka, double *state_ptr) 
   ka.exposure_en = ctx->vio_cfg.exposure_estimate_en;
   ka.state = state_ptr;
   vio_consts(ctx, ka.Rci, ka.Pci, ka.Jdp_dR);
-  ka.errors = ctx->errors.p, ka.partials = ctx->partials.p, ka.info = ctx->info.p, ka.ctrl = ctx->ctrl.p;
+  ka.errors = ctx->errors.p, ka.partials = ctx->partials.p, ka.info = ctx->info.p, ka.ctrl = &ctx->ctl.p->ctrl;
   ka.partial_stride = ctx->partial_blocks;
 }
 static int vio_grid(const esikf_ctx *ctx, int count) {
@@ -1073,18 +1089,16 @@ int esikf_vio_run(esikf_ctx *ctx, const double *state_in, const double *state_pr
     if (ctx->n_inv_refs != ctx->n_patches) return fail(ctx, ESIKF_ERR_STATE, "vio_run: inverse_composition_en needs esikf_vio_set_inverse_refs for the %d patches (have %d)", ctx->n_patches, ctx->n_inv_refs);
     if (ctx->ref_w != ctx->cam.width || ctx->ref_h != ctx->cam.height) return fail(ctx, ESIKF_ERR_STATE, "vio_run: reference images must have the camera's size");
   }
-  const bool fused_vio = ctx->n_patches > 0 && ctx->loop_mode >= 1 && (ctx->nranks == 1 || ctx->p2p) && ctx->coop_ok && ctx->coop_vio > 0 && !ctx->timing;
+  const bool fused_vio = ctx->n_patches > 0 && persistent_ok(ctx, ctx->coop_vio);
   if (!fused_vio) {
-    CK(cudaMemsetAsync(ctx->ctrl.p, 0, sizeof(Ctrl), st));
-    CK(cudaMemsetAsync(ctx->vio_stats.p, 0, sizeof(esikf_vio_stats), st));
+    CK(cudaMemsetAsync(&ctx->ctl.p->ctrl, 0, sizeof(Ctrl), st));
+    CK(cudaMemsetAsync(&ctx->ctl.p->vio_stats, 0, sizeof(esikf_vio_stats), st));
   }
   if (ctx->n_patches == 0) return ESIKF_OK;  // total_points == 0: early return (vio.cpp:786)
   VioKernelArgs ka;
-  vio_fill_args(ctx, ka, ctx->state.p);
-  SolveArgs sa;
-  memset(&sa, 0, sizeof(sa));
-  sa.state = ctx->state.p, sa.prop = ctx->prop.p, sa.info = ctx->info.p, sa.ctrl = ctx->ctrl.p;
-  sa.max_iterations = ctx->vio_cfg.max_iterations, sa.solve_mode = ctx->solve_mode, sa.vio_stats = ctx->vio_stats.p;
+  vio_fill_args(ctx, ka, ctx->state);
+  SolveArgs sa = solve_args(ctx, ctx->state, ctx->vio_cfg.max_iterations);
+  sa.vio_stats = &ctx->ctl.p->vio_stats;
   sa.old_state = ctx->old_state.p, sa.G = ctx->G.p, sa.img_point_cov = ctx->vio_cfg.img_point_cov;
   const int grid = vio_grid(ctx, ka.count);
   VioInvArgs iv;
@@ -1096,12 +1110,6 @@ int esikf_vio_run(esikf_ctx *ctx, const double *state_in, const double *state_pr
     iv.ref_w = ctx->ref_w, iv.ref_h = ctx->ref_h, iv.fx = ctx->cam.fx, iv.fy = ctx->cam.fy;
   }
   if (fused_vio) {
-    const unsigned par = ctx->launch_parity & 1;
-    unsigned int *bar = ctx->barrier.p + 64 * par, *bar_next = ctx->barrier.p + 64 * (par ^ 1);
-    unsigned long long *stamps = ctx->want_stamps ? ctx->stamps.p + 64 : nullptr;
-    if (stamps) CK(cudaMemsetAsync(stamps, 0, 512 * sizeof(unsigned long long), st));
-    size_t parity_stride = (size_t)ctx->partial_blocks * NE_MAX;
-    PeerArgs peer = peer_args(ctx);
     VioTma tma_off;
     tma_off.enabled = 0;
     VioTma *tma = &tma_off;
@@ -1110,16 +1118,9 @@ int esikf_vio_run(esikf_ctx *ctx, const double *state_in, const double *state_pr
       if (rc) return rc;
       tma = &ctx->tma;
     }
-    void *kargs[] = {(void *)&ka, (void *)&sa, (void *)&bar, (void *)&bar_next, (void *)&stamps, (void *)&parity_stride, (void *)&peer, (void *)&iv, (void *)tma};
-    const bool peers = ctx->p2p && ctx->nranks > 1;
-    const void *fn = inverse ? (peers ? (const void *)vio_update_kernel<true, true> : (const void *)vio_update_kernel<false, true>)
-                             : (peers ? (const void *)vio_update_kernel<true, false> : (const void *)vio_update_kernel<false, false>);
-    cudaError_t le = cudaLaunchCooperativeKernel(fn, dim3(grid), dim3(VIO_THREADS), kargs, VIO_PERSIST_SMEM, st);
-    if (le != cudaSuccess) return fail(ctx, ESIKF_ERR_CUDA, "cooperative launch of vio_update_kernel failed: %s", cudaGetErrorString(le));
-    ctx->launch_parity++;
-    ctx->launches += 1;
-    ctx->vio_timed = false;
-    return ESIKF_OK;
+    const void *solo = inverse ? (const void *)vio_update_kernel<false, true> : (const void *)vio_update_kernel<false, false>;
+    const void *peers = inverse ? (const void *)vio_update_kernel<true, true> : (const void *)vio_update_kernel<true, false>;
+    return launch_persistent(ctx, "vio_update_kernel", solo, peers, grid, VIO_THREADS, VIO_PERSIST_SMEM, 64, 512, &ka, &sa, &iv, tma, ctx->vio_timed);
   }
   ctx->vio_timed = ctx->timing;
   ctx->vio_slots = ctx->vio_cfg.patch_pyrimid_level * ctx->vio_cfg.max_iterations;
@@ -1154,8 +1155,8 @@ int esikf_vio_fetch(esikf_ctx *ctx, double *state_out, esikf_vio_stats *stats, f
   if (!ctx) return ESIKF_ERR_ARG;
   CK(cudaSetDevice(ctx->device));
   cudaStream_t st = ctx->stream;
-  if (state_out) CK(cudaMemcpyAsync(state_out, ctx->state.p, S_N * sizeof(double), cudaMemcpyDeviceToHost, st));
-  if (stats) CK(cudaMemcpyAsync(stats, ctx->vio_stats.p, sizeof(esikf_vio_stats), cudaMemcpyDeviceToHost, st));
+  if (state_out) CK(cudaMemcpyAsync(state_out, ctx->state, S_N * sizeof(double), cudaMemcpyDeviceToHost, st));
+  if (stats) CK(cudaMemcpyAsync(stats, &ctx->ctl.p->vio_stats, sizeof(esikf_vio_stats), cudaMemcpyDeviceToHost, st));
   if (errors && ctx->n_patches) CK(cudaMemcpyAsync(errors, ctx->errors.p, (size_t)ctx->n_patches * sizeof(float), cudaMemcpyDeviceToHost, st));
   return finish_fetch(ctx);
 }
@@ -1178,10 +1179,9 @@ int esikf_vio_get_image_patch(esikf_ctx *ctx, const double *pc, int32_t n, int32
   if (ctx->img_w == 0) return fail(ctx, ESIKF_ERR_STATE, "get_image_patch before vio_set_image");
   if (n == 0) return ESIKF_OK;
   CK(cudaSetDevice(ctx->device));
-  CK(ctx->pc_buf.reserve((size_t)n * 2));
-  CK(ctx->patch_buf.reserve((size_t)n * 64));
   cudaStream_t st = ctx->stream;
-  CK(cudaMemcpyAsync(ctx->pc_buf.p, pc, (size_t)n * 2 * sizeof(double), cudaMemcpyHostToDevice, st));
+  CK(ctx->pc_buf.upload(pc, (size_t)n * 2, (size_t)n * 2, st));
+  CK(ctx->patch_buf.reserve((size_t)n * 64));
   image_patch_kernel<<<(n * 64 + 255) / 256, 256, 0, st>>>(ctx->img.p, ctx->img_w, ctx->img_h, ctx->pc_buf.p, n, level, ctx->patch_buf.p);
   ctx->launches++;
   CK(cudaMemcpyAsync(patch_out, ctx->patch_buf.p, (size_t)n * 64 * sizeof(float), cudaMemcpyDeviceToHost, st));
@@ -1193,17 +1193,16 @@ int esikf_vio_set_ref_images(esikf_ctx *ctx, const uint8_t *const *imgs, int32_t
   if (!ctx || n_imgs < 0 || width <= 0 || height <= 0 || (n_imgs > 0 && !imgs)) return fail(ctx, ESIKF_ERR_ARG, "set_ref_images: bad argument");
   CK(cudaSetDevice(ctx->device));
   CK(cudaStreamSynchronize(ctx->stream));
-  for (uint8_t *p : ctx->ref_imgs) cudaFree(p);
   ctx->ref_imgs.clear();
   ctx->n_inv_refs = 0;  // the inverse-compositional reference indices pointed into the images just released
+  std::vector<const uint8_t *> ptrs;
   for (int i = 0; i < n_imgs; i++) {
-    uint8_t *d = nullptr;
-    CK(cudaMalloc(&d, (size_t)width * height + 64));
-    ctx->ref_imgs.push_back(d);
-    CK(cudaMemcpyAsync(d, imgs[i], (size_t)width * height, cudaMemcpyHostToDevice, ctx->stream));
+    DevBuf<uint8_t> d;
+    CK(d.upload(imgs[i], (size_t)width * height, (size_t)width * height + 64, ctx->stream));
+    ptrs.push_back(d.p);
+    ctx->ref_imgs.push_back(std::move(d));
   }
-  CK(ctx->ref_img_ptrs.reserve(n_imgs + 1));
-  if (n_imgs) CK(cudaMemcpyAsync(ctx->ref_img_ptrs.p, ctx->ref_imgs.data(), n_imgs * sizeof(uint8_t *), cudaMemcpyHostToDevice, ctx->stream));
+  CK(ctx->ref_img_ptrs.upload(ptrs.data(), n_imgs, n_imgs + 1, ctx->stream));
   CK(cudaStreamSynchronize(ctx->stream));
   ctx->ref_w = width, ctx->ref_h = height;
   return ESIKF_OK;
@@ -1216,27 +1215,21 @@ int esikf_vio_warp_patches(esikf_ctx *ctx, int32_t n, const int32_t *ref_img_ind
     return fail(ctx, ESIKF_ERR_ARG, "warp_patches: bad argument");
   if (!ctx->have_cam) return fail(ctx, ESIKF_ERR_STATE, "warp_patches before vio_set_camera");
   if (ctx->ref_imgs.empty()) return fail(ctx, ESIKF_ERR_STATE, "warp_patches before set_ref_images");
-  for (int i = 0; i < n; i++)
-    if (ref_img_index[i] < 0 || ref_img_index[i] >= (int)ctx->ref_imgs.size()) return fail(ctx, ESIKF_ERR_ARG, "warp_patches: ref image index %d", ref_img_index[i]);
+  int rc = check_ref_indices(ctx, "warp_patches", ref_img_index, n);
+  if (rc) return rc;
   if (n == 0) return ESIKF_OK;
   CK(cudaSetDevice(ctx->device));
   const int L = ctx->vio_cfg.patch_pyrimid_level;
   cudaStream_t st = ctx->stream;
-  CK(ctx->ref_idx.reserve(n));
-  CK(ctx->px_ref.reserve((size_t)n * 2));
-  CK(ctx->pos_w.reserve((size_t)n * 3));
-  CK(ctx->normal_w.reserve((size_t)n * 3));
-  CK(ctx->T_ref.reserve((size_t)n * 12));
-  CK(ctx->T_cur.reserve(12));
+  CK(ctx->ref_idx.upload(ref_img_index, n, n, st));
+  CK(ctx->px_ref.upload(px_ref, (size_t)n * 2, (size_t)n * 2, st));
+  CK(ctx->pos_w.upload(pos_w, (size_t)n * 3, (size_t)n * 3, st));
+  CK(ctx->normal_w.upload(normal_w, (size_t)n * 3, (size_t)n * 3, st));
+  CK(ctx->T_ref.upload(T_ref_w, (size_t)n * 12, (size_t)n * 12, st));
+  CK(ctx->T_cur.upload(T_cur_w, 12, 12, st));
   CK(ctx->A_cur_ref.reserve((size_t)n * 4));
   CK(ctx->search_levels.reserve(n + 1));
   CK(ctx->warp_patch.reserve((size_t)n * 64 * L + 64));
-  CK(cudaMemcpyAsync(ctx->ref_idx.p, ref_img_index, (size_t)n * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-  CK(cudaMemcpyAsync(ctx->px_ref.p, px_ref, (size_t)n * 2 * sizeof(double), cudaMemcpyHostToDevice, st));
-  CK(cudaMemcpyAsync(ctx->pos_w.p, pos_w, (size_t)n * 3 * sizeof(double), cudaMemcpyHostToDevice, st));
-  CK(cudaMemcpyAsync(ctx->normal_w.p, normal_w, (size_t)n * 3 * sizeof(double), cudaMemcpyHostToDevice, st));
-  CK(cudaMemcpyAsync(ctx->T_ref.p, T_ref_w, (size_t)n * 12 * sizeof(double), cudaMemcpyHostToDevice, st));
-  CK(cudaMemcpyAsync(ctx->T_cur.p, T_cur_w, 12 * sizeof(double), cudaMemcpyHostToDevice, st));
   CamDev cam;
   cam_dev(ctx, cam);
   warp_matrix_kernel<<<(n + 127) / 128, 128, 0, st>>>(cam, n, ctx->px_ref.p, ctx->pos_w.p, ctx->normal_w.p, ctx->T_ref.p, ctx->T_cur.p, ctx->A_cur_ref.p,
@@ -1251,11 +1244,10 @@ int esikf_vio_warp_patches(esikf_ctx *ctx, int32_t n, const int32_t *ref_img_ind
   if (keep_on_device) {
     // install as the visual sub-map of the coming update: pos = pos_w, inv_expo filled by the caller through set_patches otherwise
     CK(ctx->vis_pos.reserve((size_t)n * 3 + 4));
-    CK(ctx->inv_expo.reserve(n + 1));
     CK(ctx->errors.reserve(n + 1));
     CK(cudaMemcpyAsync(ctx->vis_pos.p, ctx->pos_w.p, (size_t)n * 3 * sizeof(double), cudaMemcpyDeviceToDevice, st));
     std::vector<double> ones(n, 1.0);
-    CK(cudaMemcpyAsync(ctx->inv_expo.p, ones.data(), (size_t)n * sizeof(double), cudaMemcpyHostToDevice, st));
+    CK(ctx->inv_expo.upload(ones.data(), n, n + 1, st));
     CK(cudaStreamSynchronize(st));
     ctx->n_patches = n;
   }
@@ -1267,23 +1259,16 @@ int esikf_vio_set_inverse_refs(esikf_ctx *ctx, int32_t n, const int32_t *ref_img
                                const double *ref_pos) {
   if (!ctx || n < 0 || (n > 0 && (!ref_img_index || !ref_px || !ref_f || !ref_R || !ref_pos))) return fail(ctx, ESIKF_ERR_ARG, "set_inverse_refs: bad argument");
   if (ctx->ref_imgs.empty() && n > 0) return fail(ctx, ESIKF_ERR_STATE, "set_inverse_refs before set_ref_images");
-  for (int i = 0; i < n; i++)
-    if (ref_img_index[i] < 0 || ref_img_index[i] >= (int)ctx->ref_imgs.size()) return fail(ctx, ESIKF_ERR_ARG, "set_inverse_refs: ref image index %d", ref_img_index[i]);
+  int rc = check_ref_indices(ctx, "set_inverse_refs", ref_img_index, n);
+  if (rc) return rc;
   CK(cudaSetDevice(ctx->device));
   cudaStream_t st = ctx->stream;
-  CK(ctx->inv_ref_idx.reserve(n + 1));
-  CK(ctx->inv_ref_px.reserve((size_t)n * 2 + 2));
-  CK(ctx->inv_ref_f.reserve((size_t)n * 3 + 3));
-  CK(ctx->inv_ref_R.reserve((size_t)n * 9 + 9));
-  CK(ctx->inv_ref_pos.reserve((size_t)n * 3 + 3));
-  if (n > 0) {
-    CK(cudaMemcpyAsync(ctx->inv_ref_idx.p, ref_img_index, (size_t)n * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(ctx->inv_ref_px.p, ref_px, (size_t)n * 2 * sizeof(double), cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(ctx->inv_ref_f.p, ref_f, (size_t)n * 3 * sizeof(double), cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(ctx->inv_ref_R.p, ref_R, (size_t)n * 9 * sizeof(double), cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(ctx->inv_ref_pos.p, ref_pos, (size_t)n * 3 * sizeof(double), cudaMemcpyHostToDevice, st));
-    CK(cudaStreamSynchronize(st));  // the caller's arrays may go away
-  }
+  CK(ctx->inv_ref_idx.upload(ref_img_index, n, n + 1, st));
+  CK(ctx->inv_ref_px.upload(ref_px, (size_t)n * 2, (size_t)n * 2 + 2, st));
+  CK(ctx->inv_ref_f.upload(ref_f, (size_t)n * 3, (size_t)n * 3 + 3, st));
+  CK(ctx->inv_ref_R.upload(ref_R, (size_t)n * 9, (size_t)n * 9 + 9, st));
+  CK(ctx->inv_ref_pos.upload(ref_pos, (size_t)n * 3, (size_t)n * 3 + 3, st));
+  if (n > 0) CK(cudaStreamSynchronize(st));  // the caller's arrays may go away
   ctx->n_inv_refs = n;
   return ESIKF_OK;
 }
@@ -1294,23 +1279,18 @@ int esikf_vio_warp_affine(esikf_ctx *ctx, int32_t n, const int32_t *ref_img_inde
     return fail(ctx, ESIKF_ERR_ARG, "warp_affine: bad argument");
   if (!ctx->have_cam) return fail(ctx, ESIKF_ERR_STATE, "warp_affine before vio_set_camera");
   if (ctx->ref_imgs.empty()) return fail(ctx, ESIKF_ERR_STATE, "warp_affine before set_ref_images");
-  for (int i = 0; i < n; i++) {
-    if (ref_img_index[i] < 0 || ref_img_index[i] >= (int)ctx->ref_imgs.size()) return fail(ctx, ESIKF_ERR_ARG, "warp_affine: ref image index %d", ref_img_index[i]);
-    if (search_level[i] < 0 || search_level[i] > 8) return fail(ctx, ESIKF_ERR_ARG, "warp_affine: search level %d", search_level[i]);
-  }
+  int rc = check_ref_indices(ctx, "warp_affine", ref_img_index, n);
+  if (!rc) rc = check_search_levels(ctx, "warp_affine", search_level, n, false);
+  if (rc) return rc;
   if (n == 0) return ESIKF_OK;
   CK(cudaSetDevice(ctx->device));
   const int L = ctx->vio_cfg.patch_pyrimid_level;
   cudaStream_t st = ctx->stream;
-  CK(ctx->ref_idx.reserve(n));
-  CK(ctx->px_ref.reserve((size_t)n * 2));
-  CK(ctx->A_cur_ref.reserve((size_t)n * 4));
-  CK(ctx->warp_levels.reserve(n + 1));
+  CK(ctx->ref_idx.upload(ref_img_index, n, n, st));
+  CK(ctx->px_ref.upload(px_ref, (size_t)n * 2, (size_t)n * 2, st));
+  CK(ctx->A_cur_ref.upload(A_cur_ref, (size_t)n * 4, (size_t)n * 4, st));
+  CK(ctx->warp_levels.upload(search_level, n, n + 1, st));
   CK(ctx->warp_out.reserve((size_t)n * 64 * L + 64));
-  CK(cudaMemcpyAsync(ctx->ref_idx.p, ref_img_index, (size_t)n * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-  CK(cudaMemcpyAsync(ctx->px_ref.p, px_ref, (size_t)n * 2 * sizeof(double), cudaMemcpyHostToDevice, st));
-  CK(cudaMemcpyAsync(ctx->A_cur_ref.p, A_cur_ref, (size_t)n * 4 * sizeof(double), cudaMemcpyHostToDevice, st));
-  CK(cudaMemcpyAsync(ctx->warp_levels.p, search_level, (size_t)n * sizeof(int32_t), cudaMemcpyHostToDevice, st));
   // separate scratch: the patches / search levels installed by set_patches (or warp_patches with keep_on_device) stay untouched
   CK(cudaMemsetAsync(ctx->warp_out.p, 0, (size_t)n * 64 * L * sizeof(float), st));
   warp_affine_kernel<<<(n * L * 64 + 255) / 256, 256, 0, st>>>(ctx->ref_img_ptrs.p, ctx->ref_idx.p, ctx->ref_w, ctx->ref_h, n, L, ctx->A_cur_ref.p,
@@ -1406,23 +1386,20 @@ int esikf_profile_kernel(esikf_ctx *ctx, int32_t which, int32_t arg, int32_t rep
   const size_t flush_bytes = 256u << 20;
   if (flush_l2) CK(ctx->flush.reserve(flush_bytes));
   // work on a scratch copy of the resident state so the measured launches never disturb an update in flight
-  CK(cudaMemcpyAsync(ctx->scratch_state.p, ctx->state.p, S_N * sizeof(double), cudaMemcpyDeviceToDevice, st));
-  CK(cudaMemsetAsync(ctx->ctrl.p, 0, sizeof(Ctrl), st));
-  cudaEvent_t e0, e1;
-  CK(cudaEventCreate(&e0));
-  CK(cudaEventCreate(&e1));
+  Ctrl *ctrl = &ctx->ctl.p->ctrl;
+  CK(cudaMemcpyAsync(ctx->scratch_state.p, ctx->state, S_N * sizeof(double), cudaMemcpyDeviceToDevice, st));
+  CK(cudaMemsetAsync(ctrl, 0, sizeof(Ctrl), st));
+  cudaEvent_t e0 = ctx->prof_ev[0], e1 = ctx->prof_ev[1];
   double total = 0.0;
   LioKernelArgs la;
   VioKernelArgs va;
-  SolveArgs sa;
-  memset(&sa, 0, sizeof(sa));
+  SolveArgs sa{};
   int grid = 1;
   if (which == 0 || which == 1 || which == 3) {
     if (!ctx->have_map || ctx->n_pts == 0 || ctx->scan_fresh) return fail(ctx, ESIKF_ERR_STATE, "profile_kernel: no resident LIO frame (run lio once)");
     lio_fill_args(ctx, la, ctx->scratch_state.p);
     grid = lio_grid(ctx, la.count);
-    sa.state = ctx->scratch_state.p, sa.prop = ctx->prop.p, sa.info = ctx->info.p, sa.ctrl = ctx->ctrl.p;
-    sa.max_iterations = 1 << 20, sa.solve_mode = ctx->solve_mode;
+    sa = solve_args(ctx, ctx->scratch_state.p, 1 << 20);
   } else if (which == 2) {
     if (ctx->n_patches == 0 || ctx->img_w == 0) return fail(ctx, ESIKF_ERR_STATE, "profile_kernel: no resident VIO frame");
     vio_fill_args(ctx, va, ctx->scratch_state.p);
@@ -1434,8 +1411,8 @@ int esikf_profile_kernel(esikf_ctx *ctx, int32_t which, int32_t arg, int32_t rep
   for (int r = 0; r < reps + 3; r++) {  // 3 warm-up launches
     if (flush_l2) CK(cudaMemsetAsync(ctx->flush.p, r & 0xff, flush_bytes, st));
     if (which == 1) {
-      CK(cudaMemcpyAsync(ctx->scratch_state.p, ctx->state.p, S_N * sizeof(double), cudaMemcpyDeviceToDevice, st));
-      CK(cudaMemsetAsync(ctx->ctrl.p, 0, sizeof(Ctrl), st));
+      CK(cudaMemcpyAsync(ctx->scratch_state.p, ctx->state, S_N * sizeof(double), cudaMemcpyDeviceToDevice, st));
+      CK(cudaMemsetAsync(ctrl, 0, sizeof(Ctrl), st));
     }
     CK(cudaEventRecord(e0, st));
     if (which == 0) lio_residual_kernel<<<grid, LIO_THREADS, sizeof(LioSmem), st>>>(la);
@@ -1450,8 +1427,6 @@ int esikf_profile_kernel(esikf_ctx *ctx, int32_t which, int32_t arg, int32_t rep
     CK(cudaEventElapsedTime(&ms, e0, e1));
     if (r >= 3) total += ms;
   }
-  cudaEventDestroy(e0);
-  cudaEventDestroy(e1);
   CK(cudaGetLastError());
   *avg_ms = (float)(total / reps);
   return ESIKF_OK;
