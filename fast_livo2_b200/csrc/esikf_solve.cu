@@ -300,22 +300,12 @@ __device__ __forceinline__ void lio_write_stats(const SolveArgs &a, SolveSmem &s
 }
 
 // One LIO gain solve + state update (src/voxel_map.cpp:462-499) by the calling block. Returns EKF_stop_flg.
-// `ctrl` is the loop-control block the routine reads and updates (global memory for the per-iteration kernels, the CTA's
-// shared-memory copy inside the persistent kernel). resident: P / poses / info are already staged in sm / io.
-// vec_ready: state_propagat (-) state_ is already in sm.vec (the persistent kernel evaluates it inside the barrier wait).
-__device__ __noinline__ bool lio_solve_block(const SolveArgs &a, SolveSmem &sm, SolveIO &io, Ctrl &ctrl, bool resident, bool vec_ready) {
+// `ctrl` is the loop-control block the routine reads and updates (the CTA's shared-memory copy). P, the poses and info are
+// staged in sm / io, state_propagat (-) state_ is in sm.vec (:470) and, in solve mode 0, gain_setup<6> has run.
+__device__ __noinline__ bool lio_solve_block(const SolveArgs &a, SolveSmem &sm, SolveIO &io, Ctrl &ctrl) {
   const int tid = threadIdx.x, lane = tid & 31;
   const int iterCount = ctrl.iter;
   const int rematch0 = ctrl.rematch_num;
-  if (!resident) {
-    solve_load(sm, io, a, false);
-    __syncthreads();
-  }
-  if (!vec_ready) {
-    if (tid >= 32 && tid < 64) boxminus_warp(io.pr, io.st, sm.vec, lane);  // vec = state_propagat (-) state_ (:470)
-    if (!resident && tid >= 64 && tid < 96 && a.solve_mode == 0) gain_setup<6>(sm, 1.0, lane);  // per-iteration launches: nothing is kept
-    __syncthreads();
-  }
   if (tid < 32) {
     unpack_info<6>(sm, io, lane);  // H^T R^-1 H, H^T R^-1 z
     double x[6], g[6];
@@ -371,17 +361,42 @@ __device__ __noinline__ bool lio_solve_block(const SolveArgs &a, SolveSmem &sm, 
   return stop;
 }
 
+// Shared memory of the stand-alone solve kernels (one launch per iteration, nothing kept between launches).
+struct SolveKernelSmem {
+  SolveSmem sm;
+  SolveIO io;
+  SolveLiteralScratch lit;
+  Ctrl ctrl;
+};
+
+// Prologue of the stand-alone solve kernels (m = 6: LIO, 7: VIO): the loop control and what the persistent kernels keep
+// resident — P, the poses and info, vec = state_propagat (-) state and, in solve mode 0, the gain invariants. A VIO level
+// that already ended (EKF_end, vio.cpp:1685) runs no solve, and on its last slot only the final covariance pass, which
+// needs neither vec nor the gain. Returns whether the solve routine runs.
+template <int m> __device__ __forceinline__ bool solve_kernel_prologue(const SolveArgs &a, SolveKernelSmem &s, double pscale) {
+  constexpr bool vio = (m == 7);
+  const int tid = threadIdx.x, lane = tid & 31;
+  if (tid == 0) s.sm.W = s.lit.W, s.sm.K = s.lit.K, s.ctrl = *a.ctrl;
+  __syncthreads();
+  const bool level_done = vio && a.slot_iter != 0 && s.ctrl.level_done;  // entering a level: EKF_end = false (vio.cpp:1527)
+  if (level_done && !a.last_slot) return false;
+  solve_load(s.sm, s.io, a, vio && a.slot_iter != 0);
+  __syncthreads();
+  if (!level_done) {
+    if (tid >= 32 && tid < 64) boxminus_warp(s.io.pr, s.io.st, s.sm.vec, lane);
+    if (tid >= 64 && tid < 96 && a.solve_mode == 0) gain_setup<m>(s.sm, pscale, lane);
+    __syncthreads();
+  }
+  return true;
+}
+
 __global__ void __launch_bounds__(SOLVE_THREADS, 1) lio_solve_kernel(const SolveArgs a) {
   if (a.ctrl->stop) return;
-  __shared__ SolveSmem sm;
-  __shared__ SolveIO io;
-  __shared__ SolveLiteralScratch lit;
-  __shared__ Ctrl ctrl;
-  if (threadIdx.x == 0) sm.W = lit.W, sm.K = lit.K, ctrl = *a.ctrl;
+  __shared__ SolveKernelSmem s;
+  solve_kernel_prologue<6>(a, s, 1.0);
+  lio_solve_block(a, s.sm, s.io, s.ctrl);
   __syncthreads();
-  lio_solve_block(a, sm, io, ctrl, false, false);
-  __syncthreads();
-  if (threadIdx.x == 0) a.ctrl->iter = ctrl.iter, a.ctrl->rematch_num = ctrl.rematch_num, a.ctrl->stop = ctrl.stop;
+  if (threadIdx.x == 0) a.ctrl->iter = s.ctrl.iter, a.ctrl->rematch_num = s.ctrl.rematch_num, a.ctrl->stop = s.ctrl.stop;
 }
 
 __device__ __forceinline__ void vio_write_stats(const SolveArgs &a, SolveSmem &sm, SolveIO &io) {
@@ -404,23 +419,13 @@ __device__ __forceinline__ void vio_write_stats(const SolveArgs &a, SolveSmem &s
 }
 
 // One VIO accept/rollback + gain solve (src/vio.cpp:1636-1685) by the calling block; on the last slot also the final
-// covariance update (:800). Returns EKF_end of the level. vec_ready as for lio_solve_block.
-__device__ __noinline__ bool vio_solve_block(const SolveArgs &a, SolveSmem &sm, SolveIO &io, Ctrl &ctrl, bool resident, bool vec_ready) {
+// covariance update (:800). Returns EKF_end of the level. Staged as for lio_solve_block (vec: :1664, gain_setup<7>); a level
+// that already ended (EKF_end) comes here on its last slot only, and then only P, the poses and old_state are read.
+__device__ __noinline__ bool vio_solve_block(const SolveArgs &a, SolveSmem &sm, SolveIO &io, Ctrl &ctrl) {
   const int tid = threadIdx.x, lane = tid & 31;
   const bool level_done_in = (a.slot_iter == 0) ? false : (ctrl.level_done != 0);   // entering a level: EKF_end = false (vio.cpp:1527)
   const float last_error_in = (a.slot_iter == 0) ? FLT_MAX : ctrl.last_error;       // :1528
   const int has_G_in = ctrl.has_G;
-  if (level_done_in && !a.last_slot) return true;
-  if (!resident) {
-    solve_load(sm, io, a, a.slot_iter != 0);
-    __syncthreads();
-  }
-  if (!vec_ready && !level_done_in) {
-    // vec = state_propagat (-) state (:1664) on warp 1
-    if (tid >= 32 && tid < 64) boxminus_warp(io.pr, io.st, sm.vec, lane);
-    if (!resident && tid >= 64 && tid < 96 && a.solve_mode == 0) gain_setup<7>(sm, 1.0 / a.img_point_cov, lane);  // per-iteration launches: nothing is kept
-    __syncthreads();
-  }
   if (tid < 32) {
     bool accepted = false, ekf_end = level_done_in;
     float error = 0.f, last_error = last_error_in;
@@ -505,17 +510,12 @@ __device__ __noinline__ bool vio_solve_block(const SolveArgs &a, SolveSmem &sm, 
 }
 
 __global__ void __launch_bounds__(SOLVE_THREADS, 1) vio_solve_kernel(const SolveArgs a) {
-  __shared__ SolveSmem sm;
-  __shared__ SolveIO io;
-  __shared__ SolveLiteralScratch lit;
-  __shared__ Ctrl ctrl;
-  if (threadIdx.x == 0) sm.W = lit.W, sm.K = lit.K, ctrl = *a.ctrl;
-  __syncthreads();
-  vio_solve_block(a, sm, io, ctrl, false, false);
+  __shared__ SolveKernelSmem s;
+  if (solve_kernel_prologue<7>(a, s, 1.0 / a.img_point_cov)) vio_solve_block(a, s.sm, s.io, s.ctrl);
   __syncthreads();
   if (threadIdx.x == 0) {
     const unsigned bc = a.ctrl->block_counter;
-    *a.ctrl = ctrl;
+    *a.ctrl = s.ctrl;
     a.ctrl->block_counter = bc;
   }
 }
